@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — LLGS hot-path benchmark (driver contract: one JSON line on stdout from rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
+
+`--dump-outputs DIR` (e.g. bench_outputs/) writes what the last timed step returned as DIR/<name>.npy, so that two builds run
+with the same arguments (hence the same inputs) can be compared output for output.
 
 A "step" is one env.step() of every env of the workload = one launch of the fused K1 kernel per GPU.
 Workload (config.workload): BASELINE configs[1] physics — SpinTorque-v0, stt_mram reference defaults, T = 300 K thermal
@@ -54,6 +57,7 @@ NCU_PIPES = {"fma": 52.0, "fma_heavy": 51.7, "xu": 66.6, "alu": 40.6, "fp64": 1.
              "warp_instructions_per_env_substep": 176.0}
 BYTES_PER_ENV_STEP = 150       # SURVEY §8(d): algorithmic HBM bytes per env-step
 FP32_LANES_PER_SM, N_SM = 128, 148
+DUMP_ROWS = 1 << 18            # --dump-outputs: envs kept from a larger batch (fixed sample), ~42 MB of .npy files
 
 
 def _peaks():
@@ -124,6 +128,21 @@ def make_actions(n, seed):
     a[:, 0] = rng.uniform(-1.1e-6, 1.1e-6, n)
     a[:, 1] = PULSE_S
     return a
+
+
+def dump_outputs(path, step_out, n):
+    """Write what env.step returned (obs, reward, terminated, truncated and the info tensors, rows = envs) as path/<name>.npy:
+    obs-shaped arrays in float32, the rest in float64, for a fixed sample of DUMP_ROWS envs (env_index.npy) when n is larger."""
+    import torch
+    obs, reward, terminated, truncated, info = step_out
+    idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    rows = torch.from_numpy(idx).to(obs.device)
+    os.makedirs(path, exist_ok=True)
+    arrays = dict(env_index=idx, obs=obs, reward=reward, terminated=terminated, truncated=truncated, **info)
+    for name, a in arrays.items():
+        if torch.is_tensor(a):
+            a = a.index_select(0, rows).cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 ENV_KW = dict(device_type="stt_mram", max_current=1.1e-6, temperature=300.0, include_thermal_fluctuations=True,
@@ -237,7 +256,11 @@ def main():
     ap.add_argument("--no-thermal", action="store_true", help="secondary workload: thermal off (301 flop/substep)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements (thermal-off, f64, probe)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -278,12 +301,17 @@ def main():
             dist.barrier()
         torch.cuda.synchronize(dev)
 
+    action_gen = torch.Generator(device=dev)
+    action_gen.manual_seed(4321 + rank)
+
     def fresh_actions(act):
-        """Random pulse sequences: a fresh current density per env and step, drawn on the device (the duration stays the
-        metric's 1 ns = 999 substeps). One torch fill kernel per step inside the timed region; not counted in gpu_launches."""
-        act[:, 0].uniform_(-1.1e-6, 1.1e-6)
+        """Random pulse sequences: a fresh current density per env and step, drawn on the device from a seeded generator, so
+        that the same arguments give the same inputs (the duration stays the metric's 1 ns = 999 substeps). One torch fill
+        kernel per step inside the timed region; not counted in gpu_launches."""
+        act[:, 0].uniform_(-1.1e-6, 1.1e-6, generator=action_gen)
 
     def timed_device_steps(env, act, steps, warmup):
+        """Device time of `steps` env steps after `warmup` untimed ones: (ms, kernel launches, what the last step returned)."""
         for _ in range(warmup):
             fresh_actions(act)
             env.step(act)
@@ -293,7 +321,7 @@ def main():
         e0.record()
         for _ in range(steps):
             fresh_actions(act)
-            env.step(act)
+            out = env.step(act)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -301,7 +329,7 @@ def main():
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t[0])
-        return ms, env.gpu_launches - l0
+        return ms, env.gpu_launches - l0, out
 
     # ---- headline: device-resident ------------------------------------------------------------------------------------
     env = SpinTorqueVectorEnv(num_envs=n_local, device=dev, dtype=tdtype, rng_seed=1234, env_offset=rank * n_local, **kw)
@@ -311,9 +339,11 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms, launches = timed_device_steps(env, act, args.steps, args.warmup)
+    ms, launches, last_step = timed_device_steps(env, act, args.steps, args.warmup)
     stats = all_reduce_stats(env.stats_tensor())          # one collective per rollout (K5): episode statistics
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step, n_local)
     sub_per_step = n_local * 999 * n_gpus
     value = sub_per_step * args.steps / (ms * 1e-3)
     env_steps = n_local * n_gpus * args.steps / (ms * 1e-3)
@@ -397,7 +427,7 @@ def main():
                                         dtype=over.get("dtype", tdtype))
                 e.reset(seed=1234)
                 a = torch.from_numpy(make_actions(n, 7)).to(dev)
-                m, _ = timed_device_steps(e, a, max(3, args.steps // 2), 3)
+                m, _, _ = timed_device_steps(e, a, max(3, args.steps // 2), 3)
                 extras[name] = n * 999 * max(3, args.steps // 2) / (m * 1e-3)
                 del e
             variant("substeps_per_s_thermal_off", n_local, include_thermal_fluctuations=False)
@@ -421,7 +451,7 @@ def main():
             env_s = SpinTorqueVectorEnv(num_envs=n_s, device=dev, dtype=tdtype, rng_seed=1234, env_offset=rank * n_s, **kw)
             env_s.reset(seed=1234)
             act_s = torch.from_numpy(make_actions(n_s, 300 + rank)).to(dev)
-            ms_s, _ = timed_device_steps(env_s, act_s, args.steps, args.warmup)
+            ms_s, _, _ = timed_device_steps(env_s, act_s, args.steps, args.warmup)
             if rank == 0:
                 extras["strong_scaling_total_1048576"] = {
                     "envs_per_gpu": n_s, "ms_per_step": ms_s / args.steps,
