@@ -536,6 +536,39 @@ int stg_vec3_op_f64(int32_t op, const double* d_a, const double* d_b, int32_t b_
 int stg_phase_diagram_f64(const double* d_currents, const double* d_fields, int32_t n_currents, int32_t n_fields, double beta,
                           double h_k, double* d_out, void* stream);
 
+/* ---- K6: generalised advantage estimation over a stored rollout ----------------------------------------------------------
+ * Replaces Stable-Baselines3's RolloutBuffer.compute_returns_and_advantage together with the TimeLimit.truncated bootstrap of
+ * OnPolicyAlgorithm.collect_rollouts (`rewards[idx] += gamma * terminal_value`), in float32 and SB3's expression order, every
+ * product and sum rounded on its own (no contraction; spin_torque_rl_gym_b200/csrc/rollout_core.cuh). Every plane is
+ * [n_steps][n_envs] row-major (time-major), device memory:
+ *   d_reward f32        the env's reward of step t
+ *   d_value f32         V(obs_t)
+ *   d_terminated u8, d_truncated u8   the step's flags (nonzero = set; both may be set)
+ *   d_final_value f32   V(final_observation_t); read only where truncated && !terminated, other entries may hold anything (NaN)
+ *   d_last_value f32 [n_envs]          V of the observation after step n_steps - 1
+ *   d_advantage f32 out; d_return f32 out (= advantage + value) or NULL
+ * With done_t = term_t | trunc_t, nnt_t = 1 - done_t, v_next = value_{t+1} (d_last_value at the last step), adv_{n_steps} = 0:
+ *   r_t = reward_t + gamma * final_value_t where trunc_t && !term_t (else reward_t)
+ *   adv_t = ((r_t + (gamma * v_next) * nnt_t) - value_t) + (gamma_lambda * nnt_t) * adv_{t+1}
+ * gamma = float32(gamma), gamma_lambda = float32(gamma * gae_lambda) with the product in double: what SB3's NumPy evaluates.
+ * Errors: args NULL -> STG_E_NULL; a negative size -> STG_E_SIZE; n_steps == 0 or n_envs == 0 -> STG_OK without a launch;
+ * then any NULL pointer except d_return -> STG_E_NULL. */
+typedef struct StgGaeArgs {
+    const float* d_reward;
+    const float* d_value;
+    const uint8_t* d_terminated;
+    const uint8_t* d_truncated;
+    const float* d_final_value;
+    const float* d_last_value;
+    float* d_advantage;
+    float* d_return;
+    float gamma;
+    float gamma_lambda;
+    int64_t n_steps;
+    int64_t n_envs;
+} StgGaeArgs;
+int stg_rollout_gae_f32(const StgGaeArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

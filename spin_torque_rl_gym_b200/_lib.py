@@ -145,6 +145,13 @@ class StgArrayStepArgs(C.Structure):
                 ("array_offset", C.c_uint64), ("n_arrays", C.c_int64), ("action_stride", C.c_int32), ("flags", C.c_uint32)]
 
 
+class StgGaeArgs(C.Structure):
+    _fields_ = [("d_reward", C.c_void_p), ("d_value", C.c_void_p), ("d_terminated", C.c_void_p),
+                ("d_truncated", C.c_void_p), ("d_final_value", C.c_void_p), ("d_last_value", C.c_void_p),
+                ("d_advantage", C.c_void_p), ("d_return", C.c_void_p), ("gamma", C.c_float),
+                ("gamma_lambda", C.c_float), ("n_steps", C.c_int64), ("n_envs", C.c_int64)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -189,6 +196,7 @@ SYMBOLS = {
                                   C.c_int64, C.c_void_p]),
     "stg_phase_diagram_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p,
                                         C.c_void_p]),
+    "stg_rollout_gae_f32": (C.c_int, [C.POINTER(StgGaeArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

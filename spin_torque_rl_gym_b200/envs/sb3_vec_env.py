@@ -6,9 +6,11 @@ same-step auto-reset, `infos[i]['terminal_observation']` and `infos[i]['TimeLimi
 subclasses stable_baselines3's VecEnv when it can be imported, so `PPO('MlpPolicy', SB3VecEnvAdapter(env))` works unchanged.
 
 For env counts where SB3's host-side rollout buffer cannot exist (n_steps=2048 x 1M envs x 12 floats = 100 TB), RolloutCollector
-keeps a [T, N, ...] ring of observations / actions / rewards / dones on the GPU with SB3-shaped tensors."""
+keeps a [T, N, ...] ring of observations / actions / rewards / dones on the GPU with SB3-shaped tensors, and optionally the values,
+log-probabilities and flags PPO needs together with the GAE advantages computed from them in one kernel."""
 from __future__ import annotations
 
+import ctypes as C
 from typing import Any, Callable, Dict, List, Optional, Sequence
 
 import numpy as np
@@ -95,21 +97,44 @@ class SB3VecEnvAdapter(_VecEnvBase):
 
 class RolloutCollector:
     """GPU-resident rollout of `n_steps` env steps: everything stays in HBM, one kernel launch per step plus the policy.
-    `policy(obs[N,12] f32 cuda) -> actions[N,2] f32 cuda` (any torch module / callable)."""
+    `policy(obs[N,12] f32 cuda) -> actions[N,2] f32 cuda` (any torch module / callable).
 
-    def __init__(self, env, n_steps: int, store_observations: bool = True):
+    `store_values=True` keeps what PPO consumes as well: `policy(obs)` then returns `(actions [N,2], values [N] or [N,1],
+    log_probs [N])` (SB3's ActorCriticPolicy.forward convention) and `collect(policy, value_fn)` stores `values`, `log_probs`,
+    the step's `terminated` / `truncated` flags, `final_values` (`value_fn` on the step's final observations, for all N rows:
+    one extra critic forward per step instead of a host synchronisation to find the ended envs) and `last_values` (`value_fn` on
+    the observation after the last step). `compute_returns_and_advantage()` then fills `advantages` and `returns` in one kernel
+    launch (K6), bootstrapping truncated episodes with V(final observation) like SB3's collect_rollouts. `rewards` stays the
+    env's reward."""
+
+    def __init__(self, env, n_steps: int, store_observations: bool = True, store_values: bool = False):
         torch = _lib.require_cuda()
         self.env, self.n_steps = env, int(n_steps)
         N, dev = env.num_envs, env.device
         self.store_observations = store_observations
+        self.store_values = store_values
+        if store_values:
+            if not env.autoreset:
+                raise ValueError("store_values=True needs an env constructed with autoreset=True (final observations)")
+            if env.host_outputs:
+                raise ValueError("store_values=True needs the env's outputs on the device (host_outputs=False)")
         if store_observations:
             self.observations = torch.empty(self.n_steps, N, _lib.OBS_DIM, dtype=torch.float32, device=dev)
         self.actions = torch.empty(self.n_steps, N, 2, dtype=torch.float32, device=dev)
         self.rewards = torch.empty(self.n_steps, N, dtype=torch.float32, device=dev)
         self.dones = torch.empty(self.n_steps, N, dtype=torch.bool, device=dev)
+        if store_values:
+            plane = lambda dtype: torch.empty(self.n_steps, N, dtype=dtype, device=dev)  # noqa: E731
+            self.values, self.log_probs, self.final_values = plane(torch.float32), plane(torch.float32), plane(torch.float32)
+            self.terminated, self.truncated = plane(torch.bool), plane(torch.bool)
+            self.last_values = torch.empty(N, dtype=torch.float32, device=dev)
+            self.advantages, self.returns = plane(torch.float32), plane(torch.float32)
+            self._values_collected = False
         self._last_obs = None
 
-    def collect(self, policy: Callable) -> Dict[str, Any]:
+    def collect(self, policy: Callable, value_fn: Optional[Callable] = None) -> Dict[str, Any]:
+        if self.store_values:
+            return self._collect_with_values(policy, value_fn)
         env = self.env
         if self._last_obs is None:
             self._last_obs, _ = env.reset()
@@ -124,3 +149,53 @@ class RolloutCollector:
             self.dones[t].copy_(term | trunc)
         self._last_obs = obs
         return all_reduce_stats(env.stats_tensor())       # one collective per rollout: episode statistics (K5)
+
+    def _collect_with_values(self, policy: Callable, value_fn: Optional[Callable]) -> Dict[str, Any]:
+        import torch
+        if value_fn is None:
+            raise ValueError("a collector with store_values=True needs collect(policy, value_fn)")
+        env, N = self.env, self.env.num_envs
+        self._values_collected = False
+        if self._last_obs is None:
+            self._last_obs, _ = env.reset()
+        obs = self._last_obs
+        with torch.no_grad():                              # like SB3's collect_rollouts: the stored planes carry no graph
+            for t in range(self.n_steps):
+                if self.store_observations:
+                    self.observations[t].copy_(obs)
+                out = policy(obs)
+                if not (isinstance(out, (tuple, list)) and len(out) == 3):
+                    raise ValueError("with store_values=True, policy(obs) must return (actions, values, log_probs)")
+                act, val, logp = out
+                self.actions[t].copy_(act)
+                self.values[t].copy_(val.reshape(N))
+                self.log_probs[t].copy_(logp.reshape(N))
+                obs, rew, term, trunc, info = env.step(self.actions[t])
+                self.rewards[t].copy_(rew)
+                self.terminated[t].copy_(term)
+                self.truncated[t].copy_(trunc)
+                self.dones[t].copy_(term | trunc)
+                # every row, ended or not: rows of envs that did not end are stale and never read by the GAE kernel
+                self.final_values[t].copy_(value_fn(info["final_observation"]).reshape(N))
+            self.last_values.copy_(value_fn(obs).reshape(N))
+        self._last_obs = obs
+        self._values_collected = True
+        return all_reduce_stats(env.stats_tensor())
+
+    def compute_returns_and_advantage(self, gamma: float = 0.99, gae_lambda: float = 0.95) -> None:
+        """GAE(gamma, gae_lambda) over the stored rollout into `advantages` and `returns` (SB3's
+        RolloutBuffer.compute_returns_and_advantage in float32, truncated episodes bootstrapped with `final_values`), one
+        launch of stg_rollout_gae_f32 on the env's current stream."""
+        if not (self.store_values and self._values_collected):
+            raise RuntimeError("compute_returns_and_advantage needs a collector with store_values=True and a collect() first")
+        torch = self.env._torch
+        a = _lib.StgGaeArgs()
+        a.d_reward, a.d_value = self.rewards.data_ptr(), self.values.data_ptr()
+        a.d_terminated, a.d_truncated = self.terminated.data_ptr(), self.truncated.data_ptr()
+        a.d_final_value, a.d_last_value = self.final_values.data_ptr(), self.last_values.data_ptr()
+        a.d_advantage, a.d_return = self.advantages.data_ptr(), self.returns.data_ptr()
+        # NumPy's `python_float * float32_array` rounds the scalar to float32 first; gamma * gae_lambda is a double product
+        a.gamma, a.gamma_lambda = float(np.float32(gamma)), float(np.float32(gamma * gae_lambda))
+        a.n_steps, a.n_envs = self.n_steps, self.env.num_envs
+        with _lib.device_guard(torch, self.env.device):
+            _lib.check(_lib.load().stg_rollout_gae_f32(C.byref(a), self.env._stream()), "stg_rollout_gae_f32")
