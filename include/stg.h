@@ -569,6 +569,46 @@ typedef struct StgGaeArgs {
 } StgGaeArgs;
 int stg_rollout_gae_f32(const StgGaeArgs* args, void* stream);
 
+/* ---- K7: one shuffled PPO minibatch gathered from a stored rollout ---------------------------------------------------------
+ * Replaces the fancy indexing of Stable-Baselines3's RolloutBuffer.get / _get_samples (`self.observations[batch_inds]`, ...)
+ * for one minibatch of a uniform random permutation of the n_steps * n_envs samples, without materialising the permutation.
+ * Source planes are the collector's time-major device planes; destinations are dense rows:
+ *   d_obs [n_steps][n_envs][12] -> d_obs_out [batch][12]     (both 16-B aligned, else STG_E_ALIGN)
+ *   d_action [n_steps][n_envs][2] -> d_action_out [batch][2] (both 8-B aligned, else STG_E_ALIGN)
+ *   d_value, d_log_prob, d_advantage, d_return [n_steps][n_envs] -> [batch]
+ * With M = n_steps * n_envs, output row k (0 <= k < batch) is a copy of sample f = rollout_permute(round_keys, M, start + k),
+ * the flat time-major index f = t * n_envs + i (spin_torque_rl_gym_b200/csrc/rollout_core.cuh): a balanced 8-round Feistel
+ * network over the smallest even number b >= 2 of bits with 2^b >= M, round r = (murmur3 fmix32(right ^ round_keys[r])) masked
+ * to b/2 bits, cycle-walked into [0, M). It is a bijection of [0, M) for every key set, so positions 0 .. M-1 taken in
+ * consecutive minibatches visit every sample exactly once. SB3 permutes the env-major flattening (i * n_steps + t) instead;
+ * for a uniform random permutation the two orders differ only by a fixed relabelling of the samples. Values are copied bit
+ * for bit, never converted. The keys come from the caller (RolloutCollector derives them from the env's seed, env_offset
+ * and the epoch), so the library needs no random state.
+ * Each (source, destination) pair is either both NULL (that plane is skipped) or both set.
+ * Errors, in this order: args NULL -> STG_E_NULL; a negative size, n_steps * n_envs overflowing or above 2^62 -> STG_E_SIZE;
+ * batch == 0 or an empty rollout -> STG_OK without a launch; start + batch > n_steps * n_envs -> STG_E_SIZE; a pair with
+ * only one pointer set, or no pair set -> STG_E_NULL; a misaligned observation or action pointer -> STG_E_ALIGN. */
+typedef struct StgMinibatchArgs {
+    const float* d_obs;
+    float* d_obs_out;
+    const float* d_action;
+    float* d_action_out;
+    const float* d_value;
+    float* d_value_out;
+    const float* d_log_prob;
+    float* d_log_prob_out;
+    const float* d_advantage;
+    float* d_advantage_out;
+    const float* d_return;
+    float* d_return_out;
+    uint32_t round_keys[8];
+    int64_t n_steps;
+    int64_t n_envs;
+    int64_t start;   /* first permutation position of this minibatch */
+    int64_t batch;   /* rows in it */
+} StgMinibatchArgs;
+int stg_rollout_minibatch_f32(const StgMinibatchArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

@@ -152,6 +152,14 @@ class StgGaeArgs(C.Structure):
                 ("gamma_lambda", C.c_float), ("n_steps", C.c_int64), ("n_envs", C.c_int64)]
 
 
+class StgMinibatchArgs(C.Structure):
+    _fields_ = [("d_obs", C.c_void_p), ("d_obs_out", C.c_void_p), ("d_action", C.c_void_p), ("d_action_out", C.c_void_p),
+                ("d_value", C.c_void_p), ("d_value_out", C.c_void_p), ("d_log_prob", C.c_void_p),
+                ("d_log_prob_out", C.c_void_p), ("d_advantage", C.c_void_p), ("d_advantage_out", C.c_void_p),
+                ("d_return", C.c_void_p), ("d_return_out", C.c_void_p), ("round_keys", C.c_uint32 * 8),
+                ("n_steps", C.c_int64), ("n_envs", C.c_int64), ("start", C.c_int64), ("batch", C.c_int64)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -197,6 +205,7 @@ SYMBOLS = {
     "stg_phase_diagram_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p,
                                         C.c_void_p]),
     "stg_rollout_gae_f32": (C.c_int, [C.POINTER(StgGaeArgs), C.c_void_p]),
+    "stg_rollout_minibatch_f32": (C.c_int, [C.POINTER(StgMinibatchArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

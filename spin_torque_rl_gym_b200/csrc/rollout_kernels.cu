@@ -1,4 +1,5 @@
-// rollout_kernels.cu — K6: generalised advantage estimation over a stored rollout (include/stg.h, stg_rollout_gae_f32).
+// rollout_kernels.cu — K6: generalised advantage estimation over a stored rollout (include/stg.h, stg_rollout_gae_f32), and
+// K7: shuffled PPO minibatches gathered from it (stg_rollout_minibatch_f32, below K6).
 // Replaces Stable-Baselines3's RolloutBuffer.compute_returns_and_advantage (a Python loop over time with NumPy over envs)
 // plus the TimeLimit.truncated bootstrap of OnPolicyAlgorithm.collect_rollouts; the arithmetic is rollout_core.cuh.
 //
@@ -104,7 +105,72 @@ __global__ void __launch_bounds__(kGaeThreads) rollout_gae_kernel(const StgGaeAr
     }
 }
 
+// K7: one PPO minibatch (stg_rollout_minibatch_f32). One output row per thread: the row's sample index comes from the keyed
+// permutation (rollout_core.cuh, pure integer arithmetic, no memory), then every requested plane is gathered. The planes are
+// dense [T][N] (x 12 / x 2), so the flat time-major index f addresses a row directly: no division into (t, i) is needed.
+// All loads of a row are issued before its first store. The reads are random, so a sample costs whole 32-B sectors: 2 for the
+// 48-B observation row (48 f is a multiple of 16, so the row never touches a third sector), 1 for the action, 1 per scalar.
+// The outputs are written with ordinary stores: the training step reads the minibatch right after, so it may stay in L2.
+constexpr int kMinibatchThreads = 256;
+
+__global__ void __launch_bounds__(kMinibatchThreads) rollout_minibatch_kernel(const StgMinibatchArgs a) {
+    const int64_t k = (int64_t)blockIdx.x * kMinibatchThreads + threadIdx.x;
+    if (k >= a.batch) return;
+    const int64_t f = rollout_permute(a.round_keys, a.n_steps * a.n_envs, a.start + k);
+    float4 o0, o1, o2;
+    float2 act;
+    float v, lp, adv, ret;
+    if (a.d_obs) {
+        const float4* src = reinterpret_cast<const float4*>(a.d_obs + f * 12);
+        o0 = __ldg(src);
+        o1 = __ldg(src + 1);
+        o2 = __ldg(src + 2);
+    }
+    if (a.d_action) act = __ldg(reinterpret_cast<const float2*>(a.d_action) + f);
+    if (a.d_value) v = __ldg(a.d_value + f);
+    if (a.d_log_prob) lp = __ldg(a.d_log_prob + f);
+    if (a.d_advantage) adv = __ldg(a.d_advantage + f);
+    if (a.d_return) ret = __ldg(a.d_return + f);
+    if (a.d_obs) {
+        float4* dst = reinterpret_cast<float4*>(a.d_obs_out + k * 12);
+        dst[0] = o0;
+        dst[1] = o1;
+        dst[2] = o2;
+    }
+    if (a.d_action) reinterpret_cast<float2*>(a.d_action_out)[k] = act;
+    if (a.d_value) a.d_value_out[k] = v;
+    if (a.d_log_prob) a.d_log_prob_out[k] = lp;
+    if (a.d_advantage) a.d_advantage_out[k] = adv;
+    if (a.d_return) a.d_return_out[k] = ret;
+}
+
 }  // namespace stg
+
+extern "C" int stg_rollout_minibatch_f32(const StgMinibatchArgs* args, void* stream) {
+    if (!args) return STG_E_NULL;
+    const StgMinibatchArgs& a = *args;
+    if (a.n_steps < 0 || a.n_envs < 0 || a.start < 0 || a.batch < 0) return STG_E_SIZE;
+    if (a.n_envs > 0 && a.n_steps > INT64_MAX / a.n_envs) return STG_E_SIZE;
+    const int64_t M = a.n_steps * a.n_envs;
+    if (M > ((int64_t)1 << 62)) return STG_E_SIZE;
+    if (a.batch == 0 || M == 0) return STG_OK;
+    if (a.start > M - a.batch) return STG_E_SIZE;
+    const void* pairs[6][2] = {{a.d_obs, a.d_obs_out},         {a.d_action, a.d_action_out},
+                               {a.d_value, a.d_value_out},     {a.d_log_prob, a.d_log_prob_out},
+                               {a.d_advantage, a.d_advantage_out}, {a.d_return, a.d_return_out}};
+    bool any = false;
+    for (const auto& p : pairs) {
+        if (!p[0] != !p[1]) return STG_E_NULL;
+        any = any || p[0];
+    }
+    if (!any) return STG_E_NULL;
+    if (((uintptr_t)a.d_obs | (uintptr_t)a.d_obs_out) & 15u) return STG_E_ALIGN;
+    if (((uintptr_t)a.d_action | (uintptr_t)a.d_action_out) & 7u) return STG_E_ALIGN;
+    const int64_t grid = (a.batch + stg::kMinibatchThreads - 1) / stg::kMinibatchThreads;
+    if (grid > 0x7fffffff) return STG_E_SIZE;
+    stg::rollout_minibatch_kernel<<<(unsigned)grid, stg::kMinibatchThreads, 0, (cudaStream_t)stream>>>(a);
+    return (int)cudaGetLastError();
+}
 
 extern "C" int stg_rollout_gae_f32(const StgGaeArgs* args, void* stream) {
     if (!args) return STG_E_NULL;

@@ -7,11 +7,12 @@ subclasses stable_baselines3's VecEnv when it can be imported, so `PPO('MlpPolic
 
 For env counts where SB3's host-side rollout buffer cannot exist (n_steps=2048 x 1M envs x 12 floats = 100 TB), RolloutCollector
 keeps a [T, N, ...] ring of observations / actions / rewards / dones on the GPU with SB3-shaped tensors, and optionally the values,
-log-probabilities and flags PPO needs together with the GAE advantages computed from them in one kernel."""
+log-probabilities and flags PPO needs together with the GAE advantages computed from them in one kernel, and the shuffled
+minibatches of RolloutBuffer.get gathered from them one kernel launch each."""
 from __future__ import annotations
 
 import ctypes as C
-from typing import Any, Callable, Dict, List, Optional, Sequence
+from typing import Any, Callable, Dict, Iterator, List, NamedTuple, Optional, Sequence
 
 import numpy as np
 
@@ -22,6 +23,45 @@ try:  # pragma: no cover - stable_baselines3 is not in the build image
     from stable_baselines3.common.vec_env import VecEnv as _VecEnvBase
 except Exception:  # noqa: BLE001
     _VecEnvBase = object
+
+try:  # pragma: no cover - stable_baselines3 is not in the build image
+    from stable_baselines3.common.type_aliases import RolloutBufferSamples
+except Exception:  # noqa: BLE001
+    class RolloutBufferSamples(NamedTuple):
+        """Field names of stable_baselines3.common.type_aliases.RolloutBufferSamples."""
+        observations: Any
+        actions: Any
+        old_values: Any
+        old_log_prob: Any
+        advantages: Any
+        returns: Any
+
+_M64 = (1 << 64) - 1
+
+
+def _splitmix64(state: int):
+    """One step of splitmix64: (next state, output)."""
+    state = (state + 0x9E3779B97F4A7C15) & _M64
+    z = state
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _M64
+    return state, z ^ (z >> 31)
+
+
+def minibatch_round_keys(rng_seed: int, env_offset: int, epoch: int) -> List[int]:
+    """The 8 round keys of the minibatch permutation of one `RolloutCollector.get()` epoch (include/stg.h,
+    stg_rollout_minibatch_f32). A pure function: each of rng_seed, env_offset, epoch (taken mod 2^64) in turn is XORed into a
+    64-bit state (initially 0) and the state replaced by splitmix64's output for it; four more splitmix64 outputs from that
+    state give keys (low 32 bits, high 32 bits) each. So a seed reproduces every epoch's permutation, and the shards of a
+    multi-GPU run (distinct env_offset) shuffle independently."""
+    state = 0
+    for word in (rng_seed, env_offset, epoch):
+        _, state = _splitmix64(state ^ (int(word) & _M64))
+    keys = []
+    for _ in range(4):
+        state, z = _splitmix64(state)
+        keys += [z & 0xFFFFFFFF, z >> 32]
+    return keys
 
 
 class SB3VecEnvAdapter(_VecEnvBase):
@@ -105,7 +145,7 @@ class RolloutCollector:
     one extra critic forward per step instead of a host synchronisation to find the ended envs) and `last_values` (`value_fn` on
     the observation after the last step). `compute_returns_and_advantage()` then fills `advantages` and `returns` in one kernel
     launch (K6), bootstrapping truncated episodes with V(final observation) like SB3's collect_rollouts. `rewards` stays the
-    env's reward."""
+    env's reward. `get(batch_size)` then yields shuffled `RolloutBufferSamples` minibatches like SB3's RolloutBuffer.get (K7)."""
 
     def __init__(self, env, n_steps: int, store_observations: bool = True, store_values: bool = False):
         torch = _lib.require_cuda()
@@ -130,6 +170,8 @@ class RolloutCollector:
             self.last_values = torch.empty(N, dtype=torch.float32, device=dev)
             self.advantages, self.returns = plane(torch.float32), plane(torch.float32)
             self._values_collected = False
+            self._advantages_computed = False
+            self._epoch = 0                                 # get() calls so far: the epoch of the next permutation
         self._last_obs = None
 
     def collect(self, policy: Callable, value_fn: Optional[Callable] = None) -> Dict[str, Any]:
@@ -155,7 +197,7 @@ class RolloutCollector:
         if value_fn is None:
             raise ValueError("a collector with store_values=True needs collect(policy, value_fn)")
         env, N = self.env, self.env.num_envs
-        self._values_collected = False
+        self._values_collected = self._advantages_computed = False
         if self._last_obs is None:
             self._last_obs, _ = env.reset()
         obs = self._last_obs
@@ -199,3 +241,49 @@ class RolloutCollector:
         a.n_steps, a.n_envs = self.n_steps, self.env.num_envs
         with _lib.device_guard(torch, self.env.device):
             _lib.check(_lib.load().stg_rollout_gae_f32(C.byref(a), self.env._stream()), "stg_rollout_gae_f32")
+        self._advantages_computed = True
+
+    def get(self, batch_size: Optional[int] = None) -> Iterator[RolloutBufferSamples]:
+        """One epoch of shuffled minibatches over the n_steps * num_envs stored samples, like SB3's RolloutBuffer.get:
+        `RolloutBufferSamples(observations [B,12], actions [B,2], old_values [B], old_log_prob [B], advantages [B],
+        returns [B])`, float32 on the env's device. `batch_size=None` yields the whole rollout as one batch; otherwise
+        consecutive slices of one permutation, the last one possibly smaller. Every call draws a new permutation: that of
+        epoch e = the number of earlier get() calls on this collector, keyed by `minibatch_round_keys(env.rng_seed,
+        env.env_offset, e)`. Each batch is one launch of stg_rollout_minibatch_f32 (K7) on the env's current stream into
+        newly allocated tensors (one allocation per batch, split into the six fields), so batches kept by the caller are
+        never overwritten; iterating never synchronises with the host. Needs store_values=True, store_observations=True
+        and compute_returns_and_advantage() after the last collect(); the arguments are checked when get() is called."""
+        if not (self.store_values and self.store_observations):
+            raise ValueError("get() needs a collector with store_values=True and store_observations=True")
+        if not self._advantages_computed:
+            raise RuntimeError("get() needs compute_returns_and_advantage() after the last collect()")
+        total = self.n_steps * self.env.num_envs
+        batch_size = total if batch_size is None else int(batch_size)
+        if batch_size <= 0:
+            raise ValueError(f"batch_size must be positive, got {batch_size}")
+        keys = minibatch_round_keys(self.env.rng_seed, self.env.env_offset, self._epoch)
+        self._epoch += 1
+        return self._minibatches(keys, batch_size)
+
+    def _minibatches(self, keys: List[int], batch_size: int) -> Iterator[RolloutBufferSamples]:
+        env = self.env
+        torch, N = env._torch, env.num_envs
+        total = self.n_steps * N
+        a = _lib.StgMinibatchArgs()
+        a.d_obs, a.d_action = self.observations.data_ptr(), self.actions.data_ptr()
+        a.d_value, a.d_log_prob = self.values.data_ptr(), self.log_probs.data_ptr()
+        a.d_advantage, a.d_return = self.advantages.data_ptr(), self.returns.data_ptr()
+        a.round_keys[:] = keys
+        a.n_steps, a.n_envs = self.n_steps, N
+        launch = _lib.load().stg_rollout_minibatch_f32
+        for start in range(0, total, batch_size):
+            B = min(batch_size, total - start)
+            with _lib.device_guard(torch, env.device):
+                buf = torch.empty(18 * B, dtype=torch.float32, device=env.device)
+                base = buf.data_ptr()           # observations first: 16-B aligned like every allocation
+                a.d_obs_out, a.d_action_out, a.d_value_out = base, base + 48 * B, base + 56 * B
+                a.d_log_prob_out, a.d_advantage_out, a.d_return_out = base + 60 * B, base + 64 * B, base + 68 * B
+                a.start, a.batch = start, B
+                _lib.check(launch(C.byref(a), env._stream()), "stg_rollout_minibatch_f32")
+            obs, act, val, logp, adv, ret = buf.split([12 * B, 2 * B, B, B, B, B])
+            yield RolloutBufferSamples(obs.view(B, _lib.OBS_DIM), act.view(B, 2), val, logp, adv, ret)
