@@ -609,6 +609,75 @@ typedef struct StgMinibatchArgs {
 } StgMinibatchArgs;
 int stg_rollout_minibatch_f32(const StgMinibatchArgs* args, void* stream);
 
+/* ---- K8: VecNormalize, running observation and return normalisation of the STT vector env -------------------------------
+ * Replaces Stable-Baselines3's VecNormalize.step_wait / reset / normalize_obs / normalize_reward with RunningMeanStd, in float64
+ * and SB3's expression order (spin_torque_rl_gym_b200/csrc/vecnorm_core.cuh). A wrapped step is three launches on one stream,
+ * with an optional gather of the moment vectors across ranks between the first two:
+ *   stg_vecnorm_moments_f32  with d_reward set: d_returns = d_returns * gamma + d_reward (two roundings). Then the moments of the
+ *                            n rows of the 12 observation columns and of the return column (zero when d_reward is NULL, which
+ *                            leaves d_returns untouched) are reduced in FP64 into d_moments[0 .. STG_VECNORM_MOMENTS).
+ *                            The reduction order is fixed: STG_VECNORM_GRID(n) CTAs write partials into d_work, the last CTA
+ *                            folds them in a fixed tree, so the bits depend only on n and the data.
+ *   stg_vecnorm_merge_f64    folds the n_ranks moment vectors d_moments [n_ranks][STG_VECNORM_MOMENTS] in rank order (Chan's
+ *                            pairwise update) and applies RunningMeanStd.update_from_moments in place to d_stats: to obs_rms when
+ *                            flags has TRAINING and NORM_OBS, to ret_rms when flags has TRAINING and d_reward is set (d_reward is
+ *                            not read). One CTA, so no CTA reads statistics another one writes.
+ *   stg_vecnorm_apply_f32    with the statistics in d_stats (not updated):
+ *                            d_obs_out = clip((d_obs - mean) / sqrt(var + epsilon), +-clip_obs) computed in f64 and rounded to f32
+ *                            (a copy without NORM_OBS); the same for the rows of d_final_obs of envs with terminated | truncated
+ *                            into d_final_obs_out (other rows are neither read nor written);
+ *                            d_reward_out = clip(d_reward / sqrt(ret_var + epsilon), +-clip_reward) (a copy without NORM_REWARD);
+ *                            d_returns of envs with terminated | truncated set to 0 (when d_returns and the flags are set).
+ *                            Each (input, output) pair may be skipped with both pointers NULL.
+ * Moment vector (doubles): [0] n, [1 + f] mean, [1 + 13 + f] M2 = sum of squared deviations, f = 0..11 observation columns, 12 the
+ * return. Statistics (doubles): obs_rms mean [0..12), var [12..24), count [24]; ret_rms mean [25], var [26], count [27]; SB3 starts
+ * them at mean 0, var 1, count 1e-4. d_work: STG_VECNORM_WORK_DOUBLES doubles whose last 8 bytes hold a CTA counter that must be
+ * zero before the first call (every call leaves it zero); it serves one stream at a time.
+ * Only the 12-float STT observation is supported. d_obs, d_final_obs and both observation outputs are 16-B aligned.
+ * Errors, in this order: args NULL -> STG_E_NULL; n_envs < 0 -> STG_E_SIZE; n_envs == 0 -> STG_OK without a launch; a
+ * required pointer NULL or a half-set pair -> STG_E_NULL; a misaligned observation pointer -> STG_E_ALIGN. The merge reads no
+ * per-env array and ignores n_envs: n_ranks < 1 -> STG_E_SIZE.
+ * Required: moments d_obs, d_moments, d_work, and d_returns with d_reward; merge d_moments, d_stats; apply d_stats, at least one
+ * pair, d_terminated and d_truncated with the final pair. */
+#define STG_VECNORM_FEATURES 13
+#define STG_VECNORM_MOMENTS 27
+#define STG_VECNORM_STATS 28
+#define STG_VECNORM_OBS_MEAN 0
+#define STG_VECNORM_OBS_VAR 12
+#define STG_VECNORM_OBS_COUNT 24
+#define STG_VECNORM_RET_MEAN 25
+#define STG_VECNORM_RET_VAR 26
+#define STG_VECNORM_RET_COUNT 27
+#define STG_VECNORM_THREADS 256
+#define STG_VECNORM_MAX_CTAS 296
+#define STG_VECNORM_GRID(n) ((n) <= 0 ? 0 : ((n) + STG_VECNORM_THREADS - 1) / STG_VECNORM_THREADS < STG_VECNORM_MAX_CTAS \
+                             ? ((n) + STG_VECNORM_THREADS - 1) / STG_VECNORM_THREADS : STG_VECNORM_MAX_CTAS)
+#define STG_VECNORM_WORK_DOUBLES (STG_VECNORM_MAX_CTAS * STG_VECNORM_MOMENTS + 1)
+#define STG_VECNORM_TRAINING 0x1u
+#define STG_VECNORM_NORM_OBS 0x2u
+#define STG_VECNORM_NORM_REWARD 0x4u
+typedef struct StgVecNormArgs {
+    const float* d_obs;              /* [n][12] raw observations                                     */
+    const float* d_final_obs;        /* [n][12] raw final observations (rows of ended envs) or NULL   */
+    const uint8_t* d_terminated;     /* [n]                                                          */
+    const uint8_t* d_truncated;      /* [n]                                                          */
+    const double* d_reward;          /* [n] raw reward or NULL                                       */
+    double* d_returns;               /* [n] discounted returns                                       */
+    double* d_stats;                 /* [STG_VECNORM_STATS]                                          */
+    double* d_moments;               /* moments: [STG_VECNORM_MOMENTS] out; merge: [n_ranks][...] in  */
+    double* d_work;                  /* [STG_VECNORM_WORK_DOUBLES]                                   */
+    float* d_obs_out;                /* [n][12]                                                      */
+    float* d_final_obs_out;          /* [n][12]                                                      */
+    double* d_reward_out;            /* [n]                                                          */
+    double gamma, epsilon, clip_obs, clip_reward;
+    int64_t n_envs;
+    int32_t n_ranks;
+    uint32_t flags;                  /* STG_VECNORM_*                                                */
+} StgVecNormArgs;
+int stg_vecnorm_moments_f32(const StgVecNormArgs* args, void* stream);
+int stg_vecnorm_merge_f64(const StgVecNormArgs* args, void* stream);
+int stg_vecnorm_apply_f32(const StgVecNormArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

@@ -31,6 +31,12 @@ SORT_WORK_INTS = 8192 + 8
 REDO_HEADER = 4          # include/stg.h STG_REDO_HEADER
 STATUS_GUARD, STATUS_INVALID_PARAMS, STATUS_REDONE_F64 = 1, 2, 4
 OBS_DIM = 12
+# K8 VecNormalize (include/stg.h STG_VECNORM_*)
+VECNORM_MOMENTS = 27      # moment vector (n, mean[13], M2[13]): 12 observation columns and the return
+VECNORM_STATS = 28        # obs_rms mean [0, 12), var [12, 24), count 24; ret_rms mean 25, var 26, count 27
+VECNORM_MAX_CTAS = 296
+VECNORM_WORK_DOUBLES = VECNORM_MAX_CTAS * VECNORM_MOMENTS + 1
+VECNORM_TRAINING, VECNORM_NORM_OBS, VECNORM_NORM_REWARD = 0x1, 0x2, 0x4
 
 
 class StgSttParams(C.Structure):
@@ -160,6 +166,15 @@ class StgMinibatchArgs(C.Structure):
                 ("n_steps", C.c_int64), ("n_envs", C.c_int64), ("start", C.c_int64), ("batch", C.c_int64)]
 
 
+class StgVecNormArgs(C.Structure):
+    _fields_ = [("d_obs", C.c_void_p), ("d_final_obs", C.c_void_p), ("d_terminated", C.c_void_p),
+                ("d_truncated", C.c_void_p), ("d_reward", C.c_void_p), ("d_returns", C.c_void_p), ("d_stats", C.c_void_p),
+                ("d_moments", C.c_void_p), ("d_work", C.c_void_p), ("d_obs_out", C.c_void_p),
+                ("d_final_obs_out", C.c_void_p), ("d_reward_out", C.c_void_p), ("gamma", C.c_double),
+                ("epsilon", C.c_double), ("clip_obs", C.c_double), ("clip_reward", C.c_double), ("n_envs", C.c_int64),
+                ("n_ranks", C.c_int32), ("flags", C.c_uint32)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -206,6 +221,9 @@ SYMBOLS = {
                                         C.c_void_p]),
     "stg_rollout_gae_f32": (C.c_int, [C.POINTER(StgGaeArgs), C.c_void_p]),
     "stg_rollout_minibatch_f32": (C.c_int, [C.POINTER(StgMinibatchArgs), C.c_void_p]),
+    "stg_vecnorm_moments_f32": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
+    "stg_vecnorm_merge_f64": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
+    "stg_vecnorm_apply_f32": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

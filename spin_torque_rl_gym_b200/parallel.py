@@ -1,6 +1,7 @@
 """Multi-GPU plumbing: the env batch shards by contiguous global env-id ranges (one process per GPU, no data-path
-collective); the only collective is one all-reduce(SUM) of the STG_NSTATS-element episode-statistics vector per rollout
-(SURVEY.md §8e — the reference analogue is the per-env EnvironmentMonitor, utils/monitoring.py:89-116)."""
+collective); one all-reduce(SUM) of the STG_NSTATS-element episode-statistics vector per rollout (SURVEY.md §8e — the
+reference analogue is the per-env EnvironmentMonitor, utils/monitoring.py:89-116), and, under a synchronised VecNormalize, one
+all-gather of the 27-double moment vector per env step (all_gather_moments)."""
 from __future__ import annotations
 
 from typing import Dict, Tuple
@@ -68,3 +69,17 @@ def all_reduce_stats(stats, group=None) -> Dict[str, float]:
     out["mean_step_energy"] = out["energy"] / out["steps"] if out["steps"] else 0.0
     out["mean_reward"] = out["reward"] / out["steps"] if out["steps"] else 0.0
     return out
+
+
+def all_gather_moments(local, group=None):
+    """[G, 27] stack of every rank's moment vector `local` [27] (float64, VecNormalize / K8), in rank order. The list form of
+    all_gather, so it serves gloo (CPU tensors) and NCCL (CUDA tensors) alike; with NCCL it is enqueued on the current stream
+    and nothing waits on the host. Without an initialised process group, or with world size 1, it returns `local[None]` and
+    issues no collective."""
+    import torch
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return local[None]
+    outs = [torch.empty_like(local) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(outs, local.contiguous(), group=group)
+    return torch.stack(outs)
