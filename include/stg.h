@@ -678,6 +678,76 @@ int stg_vecnorm_moments_f32(const StgVecNormArgs* args, void* stream);
 int stg_vecnorm_merge_f64(const StgVecNormArgs* args, void* stream);
 int stg_vecnorm_apply_f32(const StgVecNormArgs* args, void* stream);
 
+/* ---- K9: ActorCriticPolicy rollout inference (Stable-Baselines3's PPO MlpPolicy) ------------------------------------------
+ * The forward pass of SB3's ActorCriticPolicy for PPO's MlpPolicy on the 12-float observation and the 2-float action:
+ * separate actor and critic MLPs 12 -> 64 -> 64 (tanh), action_net 64 -> 2 (the Gaussian mean), value_net 64 -> 1, and a
+ * state-independent log_std. The kernels are specialised for this architecture. Arithmetic: FP32, per env
+ * (spin_torque_rl_gym_b200/csrc/policy_core.cuh):
+ *   every layer output o is acc = b[o], then acc = fma(x[k], W[k][o], acc) for k = 0, 1, ..., K-1 in that order (no split-K),
+ *   hidden outputs go through tanhf (full precision);
+ *   eps0, eps1 = box_muller(Philox4x32-10 with key (key[0], key[1]) at counter (gid lo, gid hi, draw lo, draw hi)), words 0
+ *   and 1, gid = env_offset + i (llgs_core.cuh's Philox and box_muller);
+ *   a_d = mean_d + eps_d * std_d (two roundings), or mean_d with STG_POLICY_DETERMINISTIC;
+ *   log_prob = sum over d of ((-((a_d - mean_d)^2) / (2 * std_d^2) - log_std_d) - log(sqrt(2 pi))), torch's
+ *   Normal.log_prob term by term with each operation rounded on its own and IEEE division; log_std_d = the packed LOG_SCALE;
+ *   env_action_d = lo_d + (hi_d - lo_d) * ((clip(a_d, -1, 1) + 1) / 2), each operation rounded on its own.
+ * So every env's outputs depend only on its own row, the weights and (key, gid, draw): not on n, the launch geometry or the
+ * partition of the envs over launches or GPUs.
+ *
+ * Weights: one buffer of STG_POLICY_FLOATS floats, 16-B aligned, at the offsets below. Matrices are k-major: W[k][o] (input k,
+ * output o) at W + k * n_out + o, i.e. the transpose of torch's Linear.weight [out][in]. STD = exp(log_std) and LOG_SCALE =
+ * log(STD) are computed by the caller (torch) when the buffer is packed; the last three floats are padding.
+ *
+ *   stg_policy_act_f32    reads d_obs [n][12]; writes whichever of d_obs_copy [n][12] (a copy of d_obs), d_action [n][2]
+ *                         (the raw sample), d_env_action [n][2], d_value [n], d_log_prob [n] is not NULL. d_mask is ignored.
+ *   stg_policy_value_f32  the critic only: d_value [i] = V(d_obs[i]) for every row i with d_mask[i] != 0 (u8 [n]; NULL: all
+ *                         rows). Other rows are neither read nor written. Each CTA compacts the selected rows of its windows
+ *                         before computing them, so the work scales with the number of selected rows.
+ * Errors, in this order: args NULL -> STG_E_NULL; n_envs < 0 -> STG_E_SIZE; n_envs == 0 -> STG_OK without a launch; d_obs or
+ * d_weights NULL, act without any output, value with d_value NULL -> STG_E_NULL; d_obs, d_weights or d_obs_copy not 16-B
+ * aligned, d_action or d_env_action not 8-B aligned -> STG_E_ALIGN; flags other than STG_POLICY_DETERMINISTIC -> STG_E_ENUM. */
+#define STG_POLICY_OBS 12
+#define STG_POLICY_HIDDEN 64
+#define STG_POLICY_ACTIONS 2
+#define STG_POLICY_PI_W1 0          /* [12][64]  mlp_extractor.policy_net.0.weight, transposed */
+#define STG_POLICY_PI_B1 768        /* [64]      mlp_extractor.policy_net.0.bias              */
+#define STG_POLICY_PI_W2 832        /* [64][64]  mlp_extractor.policy_net.2.weight, transposed */
+#define STG_POLICY_PI_B2 4928       /* [64]                                                   */
+#define STG_POLICY_VF_W1 4992       /* [12][64]  mlp_extractor.value_net.0.weight, transposed  */
+#define STG_POLICY_VF_B1 5760
+#define STG_POLICY_VF_W2 5824       /* [64][64]  mlp_extractor.value_net.2.weight, transposed  */
+#define STG_POLICY_VF_B2 9920
+#define STG_POLICY_ACT_W 9984       /* [64][2]   action_net.weight, transposed                 */
+#define STG_POLICY_ACT_B 10112      /* [2]                                                    */
+#define STG_POLICY_VAL_W 10114      /* [64]      value_net.weight                             */
+#define STG_POLICY_VAL_B 10178      /* [1]                                                    */
+#define STG_POLICY_LOG_STD 10179    /* [2]       log_std                                      */
+#define STG_POLICY_STD 10181        /* [2]       exp(log_std)                                 */
+#define STG_POLICY_LOG_SCALE 10183  /* [2]       log(exp(log_std))                            */
+#define STG_POLICY_PARAMS 10181     /* SB3's parameters: everything before STD                */
+#define STG_POLICY_FLOATS 10188
+#define STG_POLICY_DETERMINISTIC 0x1u
+typedef struct StgPolicyArgs {
+    const float* d_obs;              /* [n][12]                                                      */
+    const float* d_weights;          /* [STG_POLICY_FLOATS]                                          */
+    const uint8_t* d_mask;           /* value: [n] or NULL                                           */
+    float* d_obs_copy;               /* act: [n][12] or NULL                                         */
+    float* d_action;                 /* act: [n][2] or NULL                                          */
+    float* d_env_action;             /* act: [n][2] or NULL                                          */
+    float* d_value;                  /* [n]; act: or NULL                                            */
+    float* d_log_prob;               /* act: [n] or NULL                                             */
+    float action_low[2];             /* the env's action Box, for d_env_action                      */
+    float action_high[2];
+    uint32_t key[2];                 /* Philox key of the action noise                               */
+    uint64_t draw;                   /* noise draw index: one per sampling launch                    */
+    uint64_t env_offset;             /* global id of row 0                                           */
+    int64_t n_envs;
+    uint32_t flags;                  /* STG_POLICY_DETERMINISTIC                                     */
+    uint32_t reserved;
+} StgPolicyArgs;
+int stg_policy_act_f32(const StgPolicyArgs* args, void* stream);
+int stg_policy_value_f32(const StgPolicyArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

@@ -37,6 +37,13 @@ VECNORM_STATS = 28        # obs_rms mean [0, 12), var [12, 24), count 24; ret_rm
 VECNORM_MAX_CTAS = 296
 VECNORM_WORK_DOUBLES = VECNORM_MAX_CTAS * VECNORM_MOMENTS + 1
 VECNORM_TRAINING, VECNORM_NORM_OBS, VECNORM_NORM_REWARD = 0x1, 0x2, 0x4
+# K9 ActorCriticPolicy (include/stg.h STG_POLICY_*): offsets into the packed weight buffer, in floats
+POLICY_LAYOUT = {"PI_W1": 0, "PI_B1": 768, "PI_W2": 832, "PI_B2": 4928, "VF_W1": 4992, "VF_B1": 5760, "VF_W2": 5824,
+                 "VF_B2": 9920, "ACT_W": 9984, "ACT_B": 10112, "VAL_W": 10114, "VAL_B": 10178, "LOG_STD": 10179,
+                 "STD": 10181, "LOG_SCALE": 10183}
+POLICY_PARAMS = 10181
+POLICY_FLOATS = 10188
+POLICY_DETERMINISTIC = 0x1
 
 
 class StgSttParams(C.Structure):
@@ -175,6 +182,14 @@ class StgVecNormArgs(C.Structure):
                 ("n_ranks", C.c_int32), ("flags", C.c_uint32)]
 
 
+class StgPolicyArgs(C.Structure):
+    _fields_ = [("d_obs", C.c_void_p), ("d_weights", C.c_void_p), ("d_mask", C.c_void_p), ("d_obs_copy", C.c_void_p),
+                ("d_action", C.c_void_p), ("d_env_action", C.c_void_p), ("d_value", C.c_void_p), ("d_log_prob", C.c_void_p),
+                ("action_low", C.c_float * 2), ("action_high", C.c_float * 2), ("key", C.c_uint32 * 2),
+                ("draw", C.c_uint64), ("env_offset", C.c_uint64), ("n_envs", C.c_int64), ("flags", C.c_uint32),
+                ("reserved", C.c_uint32)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -224,6 +239,8 @@ SYMBOLS = {
     "stg_vecnorm_moments_f32": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
     "stg_vecnorm_merge_f64": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
     "stg_vecnorm_apply_f32": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
+    "stg_policy_act_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
+    "stg_policy_value_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

@@ -145,7 +145,11 @@ class RolloutCollector:
     one extra critic forward per step instead of a host synchronisation to find the ended envs) and `last_values` (`value_fn` on
     the observation after the last step). `compute_returns_and_advantage()` then fills `advantages` and `returns` in one kernel
     launch (K6), bootstrapping truncated episodes with V(final observation) like SB3's collect_rollouts. `rewards` stays the
-    env's reward. `get(batch_size)` then yields shuffled `RolloutBufferSamples` minibatches like SB3's RolloutBuffer.get (K7)."""
+    env's reward. `get(batch_size)` then yields shuffled `RolloutBufferSamples` minibatches like SB3's RolloutBuffer.get (K7).
+
+    `collect(policy)` with an `ActorCriticPolicy` and no `value_fn` (store_values=True) takes the fused path: per step one K9
+    launch writes the observations, raw actions, values, log-probs and the env actions, and one masked K9 critic launch
+    computes `final_values` on the rows of the envs that ended only (see `_collect_fused`)."""
 
     def __init__(self, env, n_steps: int, store_observations: bool = True, store_values: bool = False):
         torch = _lib.require_cuda()
@@ -177,6 +181,10 @@ class RolloutCollector:
     def collect(self, policy: Callable, value_fn: Optional[Callable] = None) -> Dict[str, Any]:
         if self.store_values:
             return self._collect_with_values(policy, value_fn)
+        from ..policy import ActorCriticPolicy
+        if isinstance(policy, ActorCriticPolicy):
+            raise ValueError("an ActorCriticPolicy needs a collector with store_values=True (it returns values and "
+                             "log-probabilities, and its actions are in policy units)")
         env = self.env
         if self._last_obs is None:
             self._last_obs, _ = env.reset()
@@ -194,6 +202,9 @@ class RolloutCollector:
 
     def _collect_with_values(self, policy: Callable, value_fn: Optional[Callable]) -> Dict[str, Any]:
         import torch
+        from ..policy import ActorCriticPolicy
+        if isinstance(policy, ActorCriticPolicy) and value_fn is None:
+            return self._collect_fused(policy)
         if value_fn is None:
             raise ValueError("a collector with store_values=True needs collect(policy, value_fn)")
         env, N = self.env, self.env.num_envs
@@ -220,6 +231,46 @@ class RolloutCollector:
                 # every row, ended or not: rows of envs that did not end are stale and never read by the GAE kernel
                 self.final_values[t].copy_(value_fn(info["final_observation"]).reshape(N))
             self.last_values.copy_(value_fn(obs).reshape(N))
+        self._last_obs = obs
+        self._values_collected = True
+        return all_reduce_stats(env.stats_tensor())
+
+    def _collect_fused(self, policy) -> Dict[str, Any]:
+        """The rollout of an ActorCriticPolicy: per step one stg_policy_act_f32 launch writes observations[t], actions[t]
+        (raw samples, what evaluate_actions trains on), values[t], log_probs[t] and the env actions, the env steps on those,
+        and one stg_policy_value_f32 launch computes final_values[t] on the rows of the envs that ended. The weights are
+        packed once per rollout; nothing waits on the host."""
+        env, N = self.env, self.env.num_envs
+        torch = _lib.require_cuda()
+        if torch.device(env.device) != policy.log_std.device or policy.num_envs != N:
+            raise ValueError("the policy was built for another env (device or num_envs differ)")
+        self._values_collected = self._advantages_computed = False
+        if getattr(self, "_env_actions", None) is None:      # the env actions [N,2], allocated by the first fused collect
+            self._env_actions = torch.empty(N, 2, dtype=torch.float32, device=env.device)
+        if self._last_obs is None:
+            self._last_obs, _ = env.reset()
+        obs = self._last_obs
+        lib = _lib.load()
+        with _lib.device_guard(torch, env.device):
+            w = policy.pack_weights()
+            act, val = policy._args(w, N), policy._args(w, N)
+            act.d_env_action = self._env_actions.data_ptr()
+            for t in range(self.n_steps):
+                act.d_obs = obs.data_ptr()
+                act.d_obs_copy = self.observations[t].data_ptr() if self.store_observations else None
+                act.d_action, act.d_value = self.actions[t].data_ptr(), self.values[t].data_ptr()
+                act.d_log_prob = self.log_probs[t].data_ptr()
+                policy._set_draw(act, False)
+                _lib.check(lib.stg_policy_act_f32(C.byref(act), env._stream()), "stg_policy_act_f32")
+                obs, rew, term, trunc, info = env.step(self._env_actions)
+                self.rewards[t].copy_(rew)
+                self.terminated[t].copy_(term)
+                self.truncated[t].copy_(trunc)
+                self.dones[t].copy_(term | trunc)
+                val.d_obs, val.d_mask = info["final_observation"].data_ptr(), self.dones[t].data_ptr()
+                val.d_value = self.final_values[t].data_ptr()
+                _lib.check(lib.stg_policy_value_f32(C.byref(val), env._stream()), "stg_policy_value_f32")
+            policy.predict_values(obs, out=self.last_values)
         self._last_obs = obs
         self._values_collected = True
         return all_reduce_stats(env.stats_tensor())
