@@ -748,6 +748,81 @@ typedef struct StgPolicyArgs {
 int stg_policy_act_f32(const StgPolicyArgs* args, void* stream);
 int stg_policy_value_f32(const StgPolicyArgs* args, void* stream);
 
+/* ---- K10: PPO loss and gradient of the ActorCriticPolicy (Stable-Baselines3's PPO.train() minibatch step) ---------------
+ * For one minibatch of B rows (the RolloutBufferSamples planes, device memory) and the K9 weight buffer, computes the loss of
+ * SB3's PPO.train() and its gradient with respect to every parameter: what `loss.backward()` leaves in `.grad`.
+ * Per row i, in FP32:
+ *   forward: K9's arithmetic exactly (the same fma chains in ascending k, tanhf, pol_log_prob_term), so values_i and
+ *            logp_i are bit-equal to stg_policy_act_f32's for the same weights, observation and action;
+ *   A_i = (adv_i - mean) / (std + 1e-8f) with mean = d_adv_stats[0], std = d_adv_stats[1] (each operation IEEE-rounded:
+ *         torch's `(adv - adv.mean()) / (adv.std() + 1e-8)` bit for bit), or adv_i when d_adv_stats is NULL;
+ *   ratio_i = expf(logp_i - old_log_prob_i); c_i = min(max(ratio_i, ratio_lo), ratio_hi);
+ *   pmin_i = min(A_i * ratio_i, A_i * c_i);  clipped_i = |ratio_i - 1| > clip_range;
+ *   vpred_i = values_i, or old_value_i + clamp(values_i - old_value_i, -clip_range_vf, clip_range_vf) with STG_PPO_CLIP_VF;
+ *   kl_i = (ratio_i - 1) - (logp_i - old_log_prob_i).
+ * Losses (d_losses, 6 floats, in this order; sums over rows in FP64, the rest in FP64 and rounded once):
+ *   [0] loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss   [1] policy_loss = -sum(pmin) / B
+ *   [2] value_loss = sum((return - vpred)^2) / B   [3] entropy_loss = -sum_d(float32(0.5 + 0.5 log 2 pi) + LOG_SCALE_d)
+ *   [4] approx_kl = sum(kl) / B   [5] clip_fraction = count(clipped) / B
+ * Gradient: torch autograd's rules. torch.min sends half the gradient to each side at a tie (A_i * ratio_i == A_i * c_i
+ * compared in FP32); clamp passes it on the closed interval. So d pmin / d ratio = A_i where A_i * ratio_i < A_i * c_i or
+ * (a tie with ratio_lo <= ratio_i <= ratio_hi), A_i / 2 at a tie outside it, 0 otherwise; the value clip likewise. Through
+ * ratio = exp(.), Normal.log_prob with scale = exp(log_std) and the tanh layers; the entropy adds -ent_coef to each log_std.
+ * Each layer's weight gradient is summed over a tile of STG_PPO_TILE rows in FP32 (fma chains in ascending row), the tile sums
+ * are accumulated in FP64 per CTA, and a second launch folds the STG_PPO_GRID(B) CTA partials in CTA order in FP64 and scales
+ * them by 1/B (the actor) or 2 vf_coef/B (the critic) before one rounding to FP32. No floating-point atomics: the bits of the
+ * gradient and of the losses depend only on B, the weights and the data, not on the device, the stream or the addresses.
+ *
+ * d_grad: STG_POLICY_PARAMS floats, torch's parameter layout: every parameter at the offset of its K9 buffer slot (the
+ * STG_PPO_GRAD_* offsets equal STG_POLICY_*) but with matrices in Linear.weight's [out][in] order. It is overwritten.
+ * d_work: STG_PPO_WORK_DOUBLES(B) doubles; CTA b's partial is [b * STG_PPO_PART, (b + 1) * STG_PPO_PART): gradient sums in
+ * the d_grad layout, then the four loss sums at STG_PPO_PART_LOSS (pmin, squared value error, kl, clipped count).
+ * The Python caller computes ratio_lo = float32(1 - clip_range), ratio_hi = float32(1 + clip_range) in double first.
+ * Errors, in this order: args NULL -> STG_E_NULL; batch < 1 -> STG_E_SIZE; any pointer other than d_adv_stats NULL ->
+ * STG_E_NULL; d_weights or d_obs not 16-B aligned, d_action or d_work not 8-B aligned, any other pointer not 4-B aligned ->
+ * STG_E_ALIGN; flags other than STG_PPO_CLIP_VF -> STG_E_ENUM. */
+#define STG_PPO_TILE 128
+#define STG_PPO_MAX_CTAS 296
+#define STG_PPO_GRID(b) ((b) <= 0 ? 0 : ((b) + STG_PPO_TILE - 1) / STG_PPO_TILE < STG_PPO_MAX_CTAS \
+                         ? ((b) + STG_PPO_TILE - 1) / STG_PPO_TILE : STG_PPO_MAX_CTAS)
+#define STG_PPO_PART 10192          /* doubles per CTA partial                                       */
+#define STG_PPO_PART_LOSS 10181     /* the four loss sums within a partial                           */
+#define STG_PPO_WORK_DOUBLES(b) ((int64_t)STG_PPO_GRID(b) * STG_PPO_PART)
+#define STG_PPO_LOSSES 6
+#define STG_PPO_GRAD_PI_W1 0        /* [64][12]  d mlp_extractor.policy_net.0.weight */
+#define STG_PPO_GRAD_PI_B1 768
+#define STG_PPO_GRAD_PI_W2 832      /* [64][64]  */
+#define STG_PPO_GRAD_PI_B2 4928
+#define STG_PPO_GRAD_VF_W1 4992     /* [64][12]  d mlp_extractor.value_net.0.weight  */
+#define STG_PPO_GRAD_VF_B1 5760
+#define STG_PPO_GRAD_VF_W2 5824     /* [64][64]  */
+#define STG_PPO_GRAD_VF_B2 9920
+#define STG_PPO_GRAD_ACT_W 9984     /* [2][64]   d action_net.weight             */
+#define STG_PPO_GRAD_ACT_B 10112
+#define STG_PPO_GRAD_VAL_W 10114    /* [1][64]   d value_net.weight              */
+#define STG_PPO_GRAD_VAL_B 10178
+#define STG_PPO_GRAD_LOG_STD 10179  /* [2]       d log_std                       */
+#define STG_PPO_CLIP_VF 0x1u
+typedef struct StgPpoArgs {
+    const float* d_weights;          /* [STG_POLICY_FLOATS] the K9 buffer                            */
+    const float* d_obs;              /* [B][12]                                                      */
+    const float* d_action;           /* [B][2] raw actions (policy units)                            */
+    const float* d_old_value;        /* [B]                                                          */
+    const float* d_old_log_prob;     /* [B]                                                          */
+    const float* d_advantage;        /* [B]                                                          */
+    const float* d_return;           /* [B]                                                          */
+    const float* d_adv_stats;        /* [2] mean, std of d_advantage, or NULL: no normalisation       */
+    float* d_grad;                   /* [STG_POLICY_PARAMS] out                                      */
+    float* d_losses;                 /* [STG_PPO_LOSSES] out                                         */
+    double* d_work;                  /* [STG_PPO_WORK_DOUBLES(B)]                                    */
+    float clip_range, ratio_lo, ratio_hi, clip_range_vf;
+    float ent_coef, vf_coef;
+    uint32_t flags;                  /* STG_PPO_CLIP_VF                                              */
+    uint32_t reserved;
+    int64_t batch;
+} StgPpoArgs;
+int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

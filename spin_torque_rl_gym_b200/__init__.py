@@ -14,6 +14,6 @@ from . import _lib, build, params  # noqa: F401
 from .envs import (RolloutCollector, SB3VecEnvAdapter, SpinTorqueArrayEnv, SpinTorqueArrayVectorEnv,  # noqa: F401
                    SpinTorqueEnv, SpinTorqueVectorEnv, VecNormalize, make, register_with_gymnasium)
 from .parallel import all_gather_moments, all_reduce_stats, shard_range  # noqa: F401
-from .policy import ActorCriticPolicy  # noqa: F401
+from .policy import ActorCriticPolicy, PPOLosses  # noqa: F401
 
 register_with_gymnasium()

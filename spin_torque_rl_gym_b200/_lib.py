@@ -44,6 +44,23 @@ POLICY_LAYOUT = {"PI_W1": 0, "PI_B1": 768, "PI_W2": 832, "PI_B2": 4928, "VF_W1":
 POLICY_PARAMS = 10181
 POLICY_FLOATS = 10188
 POLICY_DETERMINISTIC = 0x1
+# K10 PPO gradient (include/stg.h STG_PPO_*)
+PPO_TILE = 128
+PPO_MAX_CTAS = 296
+PPO_PART = 10192          # doubles per CTA partial: gradient sums in the d_grad layout, then the loss sums
+PPO_PART_LOSS = 10181
+PPO_LOSSES = 6
+PPO_CLIP_VF = 0x1
+
+
+def ppo_grid(batch: int) -> int:
+    """STG_PPO_GRID(batch): CTAs of stg_policy_ppo_grad_f32, a function of the batch size alone."""
+    return 0 if batch <= 0 else min((batch + PPO_TILE - 1) // PPO_TILE, PPO_MAX_CTAS)
+
+
+def ppo_work_doubles(batch: int) -> int:
+    """STG_PPO_WORK_DOUBLES(batch)."""
+    return ppo_grid(batch) * PPO_PART
 
 
 class StgSttParams(C.Structure):
@@ -190,6 +207,15 @@ class StgPolicyArgs(C.Structure):
                 ("reserved", C.c_uint32)]
 
 
+class StgPpoArgs(C.Structure):
+    _fields_ = [("d_weights", C.c_void_p), ("d_obs", C.c_void_p), ("d_action", C.c_void_p), ("d_old_value", C.c_void_p),
+                ("d_old_log_prob", C.c_void_p), ("d_advantage", C.c_void_p), ("d_return", C.c_void_p),
+                ("d_adv_stats", C.c_void_p), ("d_grad", C.c_void_p), ("d_losses", C.c_void_p), ("d_work", C.c_void_p),
+                ("clip_range", C.c_float), ("ratio_lo", C.c_float), ("ratio_hi", C.c_float), ("clip_range_vf", C.c_float),
+                ("ent_coef", C.c_float), ("vf_coef", C.c_float), ("flags", C.c_uint32), ("reserved", C.c_uint32),
+                ("batch", C.c_int64)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -241,6 +267,7 @@ SYMBOLS = {
     "stg_vecnorm_apply_f32": (C.c_int, [C.POINTER(StgVecNormArgs), C.c_void_p]),
     "stg_policy_act_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_policy_value_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
+    "stg_policy_ppo_grad_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

@@ -3,13 +3,14 @@
 `ActorCriticPolicy` has the parameters, initialisation and torch methods of SB3's ActorCriticPolicy for a Box observation and a
 Box action (net_arch pi=[64, 64], vf=[64, 64], tanh, FlattenExtractor, DiagGaussianDistribution with a state-independent
 log_std), so SB3 state dicts load into it and back. Its `forward` and `predict_values`, which a rollout calls over all N envs
-every step, run as single launches of stg_policy_act_f32 / stg_policy_value_f32 (include/stg.h); `evaluate_actions`, which PPO
-trains through, is plain torch with autograd."""
+every step, run as single launches of stg_policy_act_f32 / stg_policy_value_f32 (include/stg.h); `evaluate_actions` is plain
+torch with autograd. `ppo_backward` computes SB3's PPO.train() loss of a minibatch and writes every parameter's gradient in
+one launch of stg_policy_ppo_grad_f32 plus a fold (K10)."""
 from __future__ import annotations
 
 import ctypes as C
 import math
-from typing import Optional, Tuple
+from typing import NamedTuple, Optional, Tuple
 
 import numpy as np
 import torch
@@ -33,6 +34,23 @@ def policy_noise_key(seed: int) -> Tuple[int, int]:
         _, state = _splitmix64(state ^ (int(word) & _M64))
     _, z = _splitmix64(state)
     return z & 0xFFFFFFFF, z >> 32
+
+
+class PPOLosses(NamedTuple):
+    """The losses of one PPO minibatch with Stable-Baselines3's PPO.train() definitions, each a 0-d float32 tensor on the
+    device: loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss, approx_kl = mean((ratio - 1) - log ratio),
+    clip_fraction = mean(|ratio - 1| > clip_range)."""
+    loss: torch.Tensor
+    policy_loss: torch.Tensor
+    value_loss: torch.Tensor
+    entropy_loss: torch.Tensor
+    approx_kl: torch.Tensor
+    clip_fraction: torch.Tensor
+
+
+# the sample planes ppo_backward reads: (RolloutBufferSamples field, trailing shape, required alignment in bytes)
+_PPO_PLANES = (("observations", (_lib.OBS_DIM,), 16), ("actions", (2,), 8), ("old_values", (), 4),
+               ("old_log_prob", (), 4), ("advantages", (), 4), ("returns", (), 4))
 
 
 class MlpExtractor(nn.Module):
@@ -133,6 +151,7 @@ class ActorCriticPolicy(nn.Module):
         self._action_high = torch.as_tensor(self._high, device=self.device)
         self._packed = None
         self._pad = None
+        self._grad = None
 
     # ---- SB3's torch methods -----------------------------------------------------------------------------------------------
     def extract_features(self, obs):
@@ -253,3 +272,78 @@ class ActorCriticPolicy(nn.Module):
             a.d_mask = mask.data_ptr()
         self._launch(_lib.load().stg_policy_value_f32, a, "stg_policy_value_f32")
         return out
+
+    # ---- K10 -----------------------------------------------------------------------------------------------------------------
+    def _grad_slots(self):
+        """(parameter, offset of its gradient in the flat buffer): include/stg.h's STG_PPO_GRAD_* offsets."""
+        L, pi, vf = _lib.POLICY_LAYOUT, self.mlp_extractor.policy_net, self.mlp_extractor.value_net
+        return ((pi[0].weight, L["PI_W1"]), (pi[0].bias, L["PI_B1"]), (pi[2].weight, L["PI_W2"]), (pi[2].bias, L["PI_B2"]),
+                (vf[0].weight, L["VF_W1"]), (vf[0].bias, L["VF_B1"]), (vf[2].weight, L["VF_W2"]), (vf[2].bias, L["VF_B2"]),
+                (self.action_net.weight, L["ACT_W"]), (self.action_net.bias, L["ACT_B"]),
+                (self.value_net.weight, L["VAL_W"]), (self.value_net.bias, L["VAL_B"]), (self.log_std, L["LOG_STD"]))
+
+    def _ppo_planes(self, samples):
+        obs = samples.observations
+        n = obs.shape[0] if isinstance(obs, torch.Tensor) and obs.dim() == 2 else 0
+        if n < 1:
+            raise ValueError("ppo_backward needs samples.observations of shape [B, 12] with B >= 1, got "
+                             f"{tuple(obs.shape) if isinstance(obs, torch.Tensor) else type(obs).__name__}")
+        planes = [getattr(samples, name) for name, _, _ in _PPO_PLANES]
+        for t, (name, tail, _) in zip(planes, _PPO_PLANES):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or tuple(t.shape) != (n,) + tail:
+                got = (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t).__name__
+                raise ValueError(f"samples.{name} must be a float32 tensor of shape {(n,) + tail}, got {got}")
+        if obs.device.type != "cuda":
+            raise _lib.StgError("ActorCriticPolicy.ppo_backward needs CUDA tensors (no CPU fallback)")
+        dev = self.log_std.device
+        for i, (t, (name, _, align)) in enumerate(zip(planes, _PPO_PLANES)):
+            if t.device != dev:
+                raise ValueError(f"samples.{name} is on {t.device}, the policy on {dev}")
+            if not t.is_contiguous() or t.data_ptr() % align:
+                planes[i] = t.contiguous().clone()
+        return n, planes
+
+    def ppo_backward(self, samples, clip_range: float = 0.2, clip_range_vf: Optional[float] = None,
+                     ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = True) -> PPOLosses:
+        """SB3's PPO.train() loss of one minibatch with the current weights, and the gradient of every parameter: the result
+        of `optimizer.zero_grad(); loss.backward()`, in one launch of stg_policy_ppo_grad_f32 and its fold (K10).
+
+        `samples`: a RolloutBufferSamples as RolloutCollector.get() yields it (float32, B >= 1 rows, on the policy's device);
+        misaligned or non-contiguous planes are copied first. With `normalize_advantage` and B > 1 the advantages are
+        normalised as SB3 does, `(adv - adv.mean()) / (adv.std() + 1e-8)`, bit for bit (the mean and std by torch, the rest
+        per row in the kernel). The weights are repacked first, so an optimiser step since the last call is seen.
+
+        Every parameter's `.grad` is set to a view into one flat gradient buffer the policy owns, and that buffer is
+        OVERWRITTEN on every call: gradients are not accumulated, and a `.grad` kept from an earlier call changes. The views
+        are reassigned on every call, so `zero_grad(set_to_none=True)` between calls does no harm. Gradient clipping and the
+        optimiser step are the caller's (`torch.nn.utils.clip_grad_norm_`, `torch.optim.Adam`). Returns PPOLosses; nothing
+        is read back to the host, so early stopping on approx_kl costs the caller one synchronisation.
+        Raises StgError without CUDA, ValueError for an empty batch or planes of the wrong shape, dtype or device."""
+        n, planes = self._ppo_planes(samples)
+        dev = self.log_std.device
+        with _lib.device_guard(torch, dev):
+            w = self.pack_weights()
+            if self._grad is None or self._grad.device != dev:
+                self._grad = torch.empty(_lib.POLICY_PARAMS, dtype=torch.float32, device=dev)
+            stats = None
+            if normalize_advantage and n > 1:
+                adv = planes[4]
+                stats = torch.stack([adv.mean(), adv.std()])
+            losses = torch.empty(_lib.PPO_LOSSES, dtype=torch.float32, device=dev)
+            work = torch.empty(_lib.ppo_work_doubles(n), dtype=torch.float64, device=dev)
+            a = _lib.StgPpoArgs()
+            a.d_weights = w.data_ptr()
+            a.d_obs, a.d_action, a.d_old_value, a.d_old_log_prob, a.d_advantage, a.d_return = (t.data_ptr() for t in planes)
+            a.d_adv_stats = None if stats is None else stats.data_ptr()
+            a.d_grad, a.d_losses, a.d_work = self._grad.data_ptr(), losses.data_ptr(), work.data_ptr()
+            cr = float(clip_range)
+            a.clip_range, a.ratio_lo, a.ratio_hi = cr, 1.0 - cr, 1.0 + cr     # rounded to float32 as torch.clamp does
+            if clip_range_vf is not None:
+                a.flags = _lib.PPO_CLIP_VF
+                a.clip_range_vf = float(clip_range_vf)
+            a.ent_coef, a.vf_coef = float(ent_coef), float(vf_coef)
+            a.batch = n
+            self._launch(_lib.load().stg_policy_ppo_grad_f32, a, "stg_policy_ppo_grad_f32")
+        for p, off in self._grad_slots():
+            p.grad = self._grad[off:off + p.numel()].view_as(p)
+        return PPOLosses(*losses.unbind())
