@@ -823,6 +823,65 @@ typedef struct StgPpoArgs {
 } StgPpoArgs;
 int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream);
 
+/* ---- K11: clipped Adam step of the ActorCriticPolicy (clip_grad_norm_ + torch.optim.Adam, SB3's PPO optimiser) -----------
+ * One launch of one CTA over the STG_POLICY_PARAMS parameters in the K10 gradient layout, in this order:
+ * 1. Gate. With d_gate set and *d_gate == 0: nothing is read or written. Otherwise, with d_losses and d_log set, the K10 losses
+ *    of the minibatch are logged (in FP64): d_log[LOG_PG, LOG_VALUE, LOG_ENTROPY, LOG_CLIP] += d_losses[1, 2, 3, 5],
+ *    d_log[LOG_COUNT] += 1, d_log[LOG_EPOCH_KL] += d_losses[4], d_log[LOG_EPOCH_COUNT] += 1, d_log[LOG_LAST_LOSS] = d_losses[0].
+ *    Then, with STG_ADAM_TARGET_KL, if (double)d_losses[4] > 1.5 * target_kl: *d_gate = 0 and the update is skipped (SB3
+ *    checks approx_kl before backward() and the step; the minibatch that trips the gate is logged).
+ * 2. Clip (STG_ADAM_CLIP). sum = the FP64 sum of (double)g * (double)g over d_grad: thread t of STG_ADAM_THREADS adds the
+ *    elements t, t + STG_ADAM_THREADS, ... in ascending order (each product and sum rounded), then a tree halves the partials
+ *    (partial[t] += partial[t + h] for h = STG_ADAM_THREADS / 2, ..., 1). No atomics: the bits depend only on the gradient.
+ *    total_norm = float32(sqrt(sum)); clip_coef = float32(1 / float32(total_norm + 1e-6f)) * float32(max_grad_norm) (torch
+ *    evaluates `max_norm / t` as t.reciprocal() * max_norm); clip_coef = 1 if it is > 1 (NaN stays NaN). Every element is
+ *    multiplied by clip_coef, also when it is 1, and written back to d_grad: clip_grad_norm_'s in-place result.
+ * 3. Adam: torch.optim.Adam's single-tensor update (no weight decay, no amsgrad, not maximize). *d_step += 1.0f (float32);
+ *    s = (double)*d_step; bc1 = 1 - pow(beta1, s), bc2 = 1 - pow(beta2, s) in FP64; these scalars are rounded to float32 once:
+ *      w1 = float32(1 - beta1), b2 = float32(beta2), w2 = float32(1 - beta2), eps_f = float32(eps),
+ *      step_size = float32(lr / bc1), bc2_sqrt = float32(sqrt(bc2)).
+ *    (pow is CUDA's double pow, accurate to 2 ulp: in rare steps these two scalars may differ in their last bit from a host
+ *    evaluation with a correctly rounded pow.)
+ *    Per element, in float32 with every operation IEEE-rounded on its own (no contraction):
+ *      m = w1 < 0.5f ? m + w1 * (g - m) : g - (g - m) * (1 - w1)      (torch's lerp formula)
+ *      v = v * b2 + (w2 * g) * g                                       (mul_, then addcmul_)
+ *      denom = sqrt(v) / bc2_sqrt + eps_f
+ *      p = p - (step_size * m) / denom                                 (addcdiv_ with value = -step_size)
+ *    with g the clipped gradient. The element at offset i of the K10 layout is parameter segment s (the last STG_PPO_GRAD_*
+ *    offset <= i) and is read and written at d_param[s][i - offset_s].
+ * d_log: STG_ADAM_LOG doubles at the STG_ADAM_LOG_* slots. The caller zeroes it before the first minibatch of PPO.train() and
+ * zeroes the two per-epoch slots at the start of every epoch: SB3 logs the means of pg, value and entropy losses and clip
+ * fractions over every minibatch evaluated, approx_kl over the last epoch, and the loss of the last minibatch evaluated.
+ * Errors, in this order: args NULL -> STG_E_NULL; a d_param, d_grad, d_exp_avg, d_exp_avg_sq or d_step pointer NULL ->
+ * STG_E_NULL; a float or int32 pointer not 4-B aligned or d_log not 8-B aligned -> STG_E_ALIGN; flags other than
+ * STG_ADAM_CLIP | STG_ADAM_TARGET_KL -> STG_E_ENUM; STG_ADAM_TARGET_KL with d_losses or d_gate NULL -> STG_E_NULL. */
+#define STG_ADAM_THREADS 1024
+#define STG_ADAM_TENSORS 13        /* the parameters, in STG_PPO_GRAD_* order                         */
+#define STG_ADAM_LOG 8             /* d_log layout, below                                             */
+#define STG_ADAM_LOG_PG 0          /* sum of policy_loss over the minibatches logged                  */
+#define STG_ADAM_LOG_VALUE 1       /* sum of value_loss                                               */
+#define STG_ADAM_LOG_ENTROPY 2     /* sum of entropy_loss                                             */
+#define STG_ADAM_LOG_CLIP 3        /* sum of clip_fraction                                            */
+#define STG_ADAM_LOG_COUNT 4       /* minibatches logged                                              */
+#define STG_ADAM_LOG_EPOCH_KL 5    /* sum of approx_kl over the minibatches logged in this epoch       */
+#define STG_ADAM_LOG_EPOCH_COUNT 6 /* minibatches logged in this epoch                                */
+#define STG_ADAM_LOG_LAST_LOSS 7   /* loss of the last minibatch logged                               */
+#define STG_ADAM_CLIP 0x1u         /* clip the global L2 norm to max_grad_norm                        */
+#define STG_ADAM_TARGET_KL 0x2u    /* gate on d_losses[4] (approx_kl) > 1.5 * target_kl               */
+typedef struct StgAdamArgs {
+    float* d_param[STG_ADAM_TENSORS];  /* each parameter's own contiguous storage (the nn.Parameter data) */
+    float* d_grad;                     /* [STG_POLICY_PARAMS] K10 layout; clipped in place, as clip_grad_norm_ does */
+    float* d_exp_avg;                  /* [STG_POLICY_PARAMS] */
+    float* d_exp_avg_sq;               /* [STG_POLICY_PARAMS] */
+    float* d_step;                     /* [1] Adam's step count, float32 as torch keeps it */
+    const float* d_losses;             /* [STG_PPO_LOSSES] K10's losses of this minibatch, or NULL */
+    int32_t* d_gate;                   /* [1] 1 open / 0 closed, or NULL */
+    double* d_log;                     /* [STG_ADAM_LOG] or NULL */
+    double lr, beta1, beta2, eps, max_grad_norm, target_kl;
+    uint32_t flags, reserved;
+} StgAdamArgs;
+int stg_policy_adam_f32(const StgAdamArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

@@ -15,5 +15,7 @@ from .envs import (RolloutCollector, SB3VecEnvAdapter, SpinTorqueArrayEnv, SpinT
                    SpinTorqueEnv, SpinTorqueVectorEnv, VecNormalize, make, register_with_gymnasium)
 from .parallel import all_gather_moments, all_reduce_stats, shard_range  # noqa: F401
 from .policy import ActorCriticPolicy, PPOLosses  # noqa: F401
+from .optim import ClippedAdam  # noqa: F401
+from .ppo import PPO  # noqa: F401
 
 register_with_gymnasium()

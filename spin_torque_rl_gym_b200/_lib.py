@@ -51,6 +51,12 @@ PPO_PART = 10192          # doubles per CTA partial: gradient sums in the d_grad
 PPO_PART_LOSS = 10181
 PPO_LOSSES = 6
 PPO_CLIP_VF = 0x1
+# K11 clipped Adam (include/stg.h STG_ADAM_*)
+ADAM_THREADS = 1024
+ADAM_TENSORS = 13
+ADAM_LOG = 8
+ADAM_LOG_SLOTS = {"PG": 0, "VALUE": 1, "ENTROPY": 2, "CLIP": 3, "COUNT": 4, "EPOCH_KL": 5, "EPOCH_COUNT": 6, "LAST_LOSS": 7}
+ADAM_CLIP, ADAM_TARGET_KL = 0x1, 0x2
 
 
 def ppo_grid(batch: int) -> int:
@@ -216,6 +222,13 @@ class StgPpoArgs(C.Structure):
                 ("batch", C.c_int64)]
 
 
+class StgAdamArgs(C.Structure):
+    _fields_ = [("d_param", C.c_void_p * ADAM_TENSORS), ("d_grad", C.c_void_p), ("d_exp_avg", C.c_void_p),
+                ("d_exp_avg_sq", C.c_void_p), ("d_step", C.c_void_p), ("d_losses", C.c_void_p), ("d_gate", C.c_void_p),
+                ("d_log", C.c_void_p), ("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
+                ("max_grad_norm", C.c_double), ("target_kl", C.c_double), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -268,6 +281,7 @@ SYMBOLS = {
     "stg_policy_act_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_policy_value_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_policy_ppo_grad_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p]),
+    "stg_policy_adam_f32": (C.c_int, [C.POINTER(StgAdamArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

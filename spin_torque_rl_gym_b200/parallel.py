@@ -60,8 +60,13 @@ def all_reduce_stats(stats, group=None) -> Dict[str, float]:
     t = stats.clone()
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
-    vals = t.detach().to("cpu", torch.float64).tolist()
-    out = dict(zip(_lib.STAT_NAMES, vals))
+    return episode_metrics(dict(zip(_lib.STAT_NAMES, t.detach().to("cpu", torch.float64).tolist())))
+
+
+def episode_metrics(totals: Dict[str, float]) -> Dict[str, float]:
+    """The statistics `totals` (one value per STAT_NAMES entry, e.g. the difference of two readings) with the derived episode
+    metrics added: episodes, success_rate, mean_episode_length, mean_step_energy and mean_reward (per step)."""
+    out = dict(totals)
     episodes = out["terminated"] + out["truncated"]
     out["episodes"] = episodes
     out["success_rate"] = out["terminated"] / episodes if episodes else 0.0
