@@ -823,6 +823,53 @@ typedef struct StgPpoArgs {
 } StgPpoArgs;
 int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream);
 
+/* ---- K12: data-parallel PPO minibatch, the K10 gradient and the advantage statistics folded across ranks in rank order -----
+ * G ranks each hold one local minibatch of a global minibatch (their union). Each rank computes FP64 vectors of its own rows,
+ * every rank gathers all G vectors (an all_gather: the same bytes everywhere, whatever the collective's algorithm), and every
+ * rank folds them left to right in rank order. So every rank ends with the same bits, and those depend only on the per-rank
+ * data and its order: not on the backend, the device, the stream or the addresses. Per minibatch, in stream order:
+ *   stg_ppo_adv_moments_f64   (n, mean, M2 = sum of squared deviations) of the n raw advantages of the local minibatch into
+ *                             d_out[3], in FP64. One CTA of STG_PPO_ADV_THREADS threads: thread t sums the rows t, t + T, ...
+ *                             shifted by its first row (K8's scheme), then the per-thread moments merge by Chan's update in a
+ *                             fixed tree (warp shuffles, then the 32 warp vectors by warp 0). No atomics. n == 0 writes
+ *                             (0, 0, 0).
+ *   stg_ppo_adv_merge_f32     folds d_moments [ranks][3] in rank order, left to right from (0, 0, 0), with Chan's update (K8's
+ *                             vn_chan_weights / vn_chan_feature), and writes d_stats[0] = float32(mean) and d_stats[1] =
+ *                             float32(sqrt(M2 / (n - 1))), each rounded once (torch's adv.mean() and adv.std(), correction 1;
+ *                             the FP64 division and square root are IEEE-rounded). A global count of 1 gives a NaN std, and a
+ *                             count of 0 a NaN mean and std, as in torch. d_stats is the d_adv_stats that K10 reads.
+ *   stg_policy_ppo_sums_f32   K10's gradient kernel on the local minibatch (args->batch rows, normalised with args->d_adv_stats),
+ *                             then a fold that writes the UNSCALED sums of the CTA partials, each slot summed in CTA order from
+ *                             0.0 as K10's fold does, into d_sums[STG_PPO_PART]: the gradient sums in the d_grad layout, the
+ *                             four loss sums at STG_PPO_PART_LOSS, the row count (double)args->batch at STG_PPO_PART_COUNT, and
+ *                             0.0 in the remaining slots. d_grad and d_losses are not used and may be NULL.
+ *   stg_policy_ppo_finish_f32 folds d_sums [ranks][STG_PPO_PART] slot by slot in rank order, left to right from 0.0, in FP64, and
+ *                             applies K10's scaling to the result with B = the folded count slot (args->batch is not read): the
+ *                             same code as K10's fold, so d_grad and d_losses follow the K10 contract above for the union
+ *                             batch. Only d_weights (for the entropy), d_grad, d_losses, ent_coef and vf_coef are read.
+ * With ranks = 1, sums then finish give d_grad and d_losses bit-equal to stg_policy_ppo_grad_f32 on the same arguments (a fold
+ * of one vector from 0.0 is exact). Across G > 1 ranks the result is the whole-batch K10 gradient up to summation order: where
+ * every rank's rows are whole STG_PPO_TILE tiles of the whole batch, the FP32 tile sums are the same and only their FP64 order
+ * differs; elsewhere the tiles themselves are cut differently.
+ * Bytes exchanged per minibatch and rank: 3 + STG_PPO_PART doubles (81,560 B).
+ * Errors, in this order:
+ *   adv_moments: n < 0 -> STG_E_SIZE; d_out NULL, or d_adv NULL with n > 0 -> STG_E_NULL; d_adv not 4-B or d_out not 8-B
+ *                aligned -> STG_E_ALIGN.
+ *   adv_merge:   ranks < 1 -> STG_E_SIZE; d_moments or d_stats NULL -> STG_E_NULL; d_moments not 8-B or d_stats not 4-B
+ *                aligned -> STG_E_ALIGN.
+ *   sums:        args NULL -> STG_E_NULL; batch < 1 -> STG_E_SIZE; d_weights, a sample plane, d_work or d_sums NULL ->
+ *                STG_E_NULL; the alignments of stg_policy_ppo_grad_f32, d_sums not 8-B aligned -> STG_E_ALIGN; flags other than
+ *                STG_PPO_CLIP_VF -> STG_E_ENUM. d_work holds STG_PPO_WORK_DOUBLES(batch) doubles, as for K10.
+ *   finish:      args NULL -> STG_E_NULL; ranks < 1 -> STG_E_SIZE; d_weights, d_grad, d_losses or d_sums NULL -> STG_E_NULL;
+ *                d_weights not 16-B, d_sums not 8-B, d_grad or d_losses not 4-B aligned -> STG_E_ALIGN. */
+#define STG_PPO_PART_COUNT 10185    /* the row count within a sums vector                            */
+#define STG_PPO_ADV_MOMENTS 3       /* (n, mean, M2)                                                 */
+#define STG_PPO_ADV_THREADS 1024
+int stg_policy_ppo_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream);
+int stg_policy_ppo_finish_f32(const StgPpoArgs* args, const double* d_sums, int32_t ranks, void* stream);
+int stg_ppo_adv_moments_f64(const float* d_adv, int64_t n, double* d_out, void* stream);
+int stg_ppo_adv_merge_f32(const double* d_moments, int32_t ranks, float* d_stats, void* stream);
+
 /* ---- K11: clipped Adam step of the ActorCriticPolicy (clip_grad_norm_ + torch.optim.Adam, SB3's PPO optimiser) -----------
  * One launch of one CTA over the STG_POLICY_PARAMS parameters in the K10 gradient layout, in this order:
  * 1. Gate. With d_gate set and *d_gate == 0: nothing is read or written. Otherwise, with d_losses and d_log set, the K10 losses

@@ -51,6 +51,10 @@ PPO_PART = 10192          # doubles per CTA partial: gradient sums in the d_grad
 PPO_PART_LOSS = 10181
 PPO_LOSSES = 6
 PPO_CLIP_VF = 0x1
+# K12 data-parallel PPO (include/stg.h)
+PPO_PART_COUNT = 10185    # the row count within a sums vector
+PPO_ADV_MOMENTS = 3       # (n, mean, M2) of the raw advantages
+PPO_ADV_THREADS = 1024
 # K11 clipped Adam (include/stg.h STG_ADAM_*)
 ADAM_THREADS = 1024
 ADAM_TENSORS = 13
@@ -281,6 +285,10 @@ SYMBOLS = {
     "stg_policy_act_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_policy_value_f32": (C.c_int, [C.POINTER(StgPolicyArgs), C.c_void_p]),
     "stg_policy_ppo_grad_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p]),
+    "stg_policy_ppo_sums_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p, C.c_void_p]),
+    "stg_policy_ppo_finish_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p, C.c_int32, C.c_void_p]),
+    "stg_ppo_adv_moments_f64": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "stg_ppo_adv_merge_f32": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "stg_policy_adam_f32": (C.c_int, [C.POINTER(StgAdamArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }

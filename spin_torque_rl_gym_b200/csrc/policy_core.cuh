@@ -12,6 +12,7 @@
 #include <math.h>
 
 #include "llgs_core.cuh"
+#include "vecnorm_core.cuh"
 #include "../../include/stg.h"
 
 namespace stg {
@@ -181,6 +182,40 @@ STG_HD void pol_ppo_losses(const double* sums, const float* w, int64_t batch, fl
     out[3] = (float)el;
     out[4] = (float)(sums[kPpoKl] / n);
     out[5] = (float)(sums[kPpoClipped] / n);
+}
+
+// ---- K12: advantage statistics across ranks (include/stg.h, stg_ppo_adv_moments_f64 / stg_ppo_adv_merge_f32) -------------
+// Moment vectors (n, mean, M2) of the raw advantages, merged with K8's Chan update (vecnorm_core.cuh).
+
+// the moments of adv[begin], adv[begin + stride], ... below n: sums shifted by the first of those rows, as K8's threads do
+STG_HD void pol_adv_moments(const float* adv, int64_t begin, int64_t n, int64_t stride, double out[3]) {
+    double cnt = 0.0, s1 = 0.0, s2 = 0.0;
+    const double x0 = begin < n ? (double)adv[begin] : 0.0;
+    for (int64_t i = begin; i < n; i += stride) {
+        const double d = (double)adv[i] - x0;
+        s1 += d;
+        s2 += d * d;
+        cnt += 1.0;
+    }
+    out[0] = cnt;
+    vn_shifted_to_moments(cnt, x0, s1, s2, out[1], out[2]);
+}
+
+// a <- a (+) b, a the left operand
+STG_HD void pol_adv_merge(double a[3], const double b[3]) {
+    double w, c;
+    vn_chan_weights(a[0], b[0], w, c);
+    vn_chan_feature(a[1], a[2], b[1], b[2], w, c);
+    a[0] = a[0] + b[0];
+}
+
+// the fold of stg_ppo_adv_merge_f32: `ranks` moment vectors in rank order, then torch's mean and std (correction 1)
+STG_HD void pol_adv_stats(const double* moments, int ranks, float out[2]) {
+    double acc[3] = {0.0, 0.0, 0.0};
+    for (int r = 0; r < ranks; ++r) pol_adv_merge(acc, moments + 3 * (int64_t)r);
+    const double n = acc[0];
+    out[0] = n > 0.0 ? (float)acc[1] : NAN;
+    out[1] = n > 0.0 ? (float)dsqrt(ddiv(acc[2], dadd(n, -1.0))) : NAN;   // n = 1: 0 / 0
 }
 
 // One row's forward pass (K9's chains) and backward pass on the host: adds its unscaled gradient to grad (the d_grad layout)

@@ -468,21 +468,78 @@ __global__ void __launch_bounds__(kPolThreads, 2) policy_ppo_grad_kernel(const S
     }
 }
 
-// Sums the CTA partials in CTA order, scales them (pol_ppo_grad_value) and writes d_grad; the last thread writes the losses.
-__global__ void __launch_bounds__(kPolThreads) policy_ppo_fold_kernel(const StgPpoArgs a, int parts) {
-    const int p = blockIdx.x * kPolThreads + threadIdx.x;
-    if (p < STG_POLICY_PARAMS) {
-        double t = 0.0;
+// slot p of `parts` vectors of STG_PPO_PART doubles, summed in vector order from 0.0
+__device__ __forceinline__ double ppo_fold_slot(const double* vecs, int parts, int p) {
+    double t = 0.0;
 #pragma unroll 8
-        for (int b = 0; b < parts; ++b) t += __ldcg(a.d_work + (int64_t)b * STG_PPO_PART + p);
-        a.d_grad[p] = pol_ppo_grad_value(p, t, a.batch, a.ent_coef, a.vf_coef);
-    } else if (p == STG_POLICY_PARAMS) {
-        double t[4] = {0.0, 0.0, 0.0, 0.0};
-        for (int b = 0; b < parts; ++b)
-#pragma unroll
-            for (int k = 0; k < 4; ++k) t[k] += __ldcg(a.d_work + (int64_t)b * STG_PPO_PART + STG_PPO_PART_LOSS + k);
-        pol_ppo_losses(t, a.d_weights, a.batch, a.ent_coef, a.vf_coef, a.d_losses);
+    for (int b = 0; b < parts; ++b) t += __ldcg(vecs + (int64_t)b * STG_PPO_PART + p);
+    return t;
+}
+
+enum PpoFold { kFoldScale, kFoldRaw, kFoldRanks };
+
+// The fold of K10 and K12 over `parts` vectors of STG_PPO_PART doubles (K10's CTA partials, or K12's per-rank sums):
+//   kFoldScale  sums in vector order, scales them (pol_ppo_grad_value, pol_ppo_losses) with B = a.batch into d_grad and
+//               d_losses: stg_policy_ppo_grad_f32;
+//   kFoldRaw    writes the same sums unscaled, with the row count a.batch, into `raw`: stg_policy_ppo_sums_f32;
+//   kFoldRanks  as kFoldScale with B = the folded count slot: stg_policy_ppo_finish_f32.
+template <PpoFold kMode>
+__global__ void __launch_bounds__(kPolThreads) policy_ppo_fold_kernel(const StgPpoArgs a, const double* vecs, int parts,
+                                                                     double* raw) {
+    const int p = blockIdx.x * kPolThreads + threadIdx.x;
+    if (p > STG_POLICY_PARAMS) return;
+    const int64_t batch = kMode == kFoldRanks ? (int64_t)ppo_fold_slot(vecs, parts, STG_PPO_PART_COUNT) : a.batch;
+    if (p < STG_POLICY_PARAMS) {
+        const double t = ppo_fold_slot(vecs, parts, p);
+        if (kMode == kFoldRaw) raw[p] = t;
+        else a.d_grad[p] = pol_ppo_grad_value(p, t, batch, a.ent_coef, a.vf_coef);
+        return;
     }
+    double t[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) t[k] = ppo_fold_slot(vecs, parts, STG_PPO_PART_LOSS + k);
+    if (kMode == kFoldRaw) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) raw[STG_PPO_PART_LOSS + k] = t[k];
+        raw[STG_PPO_PART_COUNT] = (double)a.batch;
+        for (int k = STG_PPO_PART_COUNT + 1; k < STG_PPO_PART; ++k) raw[k] = 0.0;
+    } else {
+        pol_ppo_losses(t, a.d_weights, batch, a.ent_coef, a.vf_coef, a.d_losses);
+    }
+}
+
+// K12: the advantage moments of one local minibatch, one CTA (include/stg.h). Chan merge of this lane's vector with the one
+// `off` lanes up, a shuffle-down tree: lane 0 ends with the warp's vector.
+constexpr int kAdvThreads = STG_PPO_ADV_THREADS;
+static_assert(STG_PPO_ADV_MOMENTS == 3 && kAdvThreads == 32 * 32, "stg.h and the K12 moments tree disagree");
+
+__device__ __forceinline__ void ppo_adv_warp_merge(double v[3]) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const double b[3] = {__shfl_down_sync(0xffffffffu, v[0], off), __shfl_down_sync(0xffffffffu, v[1], off),
+                             __shfl_down_sync(0xffffffffu, v[2], off)};
+        pol_adv_merge(v, b);
+    }
+}
+
+__global__ void __launch_bounds__(kAdvThreads) ppo_adv_moments_kernel(const float* __restrict__ adv, int64_t n,
+                                                                      double* out) {
+    __shared__ double sm[32][3];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double v[3];
+    pol_adv_moments(adv, threadIdx.x, n, kAdvThreads, v);
+    ppo_adv_warp_merge(v);
+    if (lane == 0) sm[warp][0] = v[0], sm[warp][1] = v[1], sm[warp][2] = v[2];
+    __syncthreads();
+    if (warp == 0) {
+        v[0] = sm[lane][0], v[1] = sm[lane][1], v[2] = sm[lane][2];
+        ppo_adv_warp_merge(v);
+        if (lane == 0) out[0] = v[0], out[1] = v[1], out[2] = v[2];
+    }
+}
+
+__global__ void __launch_bounds__(32) ppo_adv_merge_kernel(const double* moments, int ranks, float* stats) {
+    if (threadIdx.x == 0) pol_adv_stats(moments, ranks, stats);
 }
 
 struct PolLaunch {
@@ -554,25 +611,79 @@ extern "C" int stg_policy_value_f32(const StgPolicyArgs* args, void* stream) {
     return (int)cudaGetLastError();
 }
 
-extern "C" int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream) {
-    if (!args) return STG_E_NULL;
-    const StgPpoArgs& a = *args;
+namespace stg {
+
+// K10's argument checks, with the gradient and loss outputs required or not (K12's sums)
+static int ppo_check(const StgPpoArgs& a, bool outputs) {
     if (a.batch < 1) return STG_E_SIZE;
     if (!a.d_weights || !a.d_obs || !a.d_action || !a.d_old_value || !a.d_old_log_prob || !a.d_advantage || !a.d_return ||
-        !a.d_grad || !a.d_losses || !a.d_work)
+        (outputs && (!a.d_grad || !a.d_losses)) || !a.d_work)
         return STG_E_NULL;
     if (((uintptr_t)a.d_weights | (uintptr_t)a.d_obs) & 15u) return STG_E_ALIGN;
     if (((uintptr_t)a.d_action | (uintptr_t)a.d_work) & 7u) return STG_E_ALIGN;
     if (((uintptr_t)a.d_old_value | (uintptr_t)a.d_old_log_prob | (uintptr_t)a.d_advantage | (uintptr_t)a.d_return |
          (uintptr_t)a.d_adv_stats | (uintptr_t)a.d_grad | (uintptr_t)a.d_losses) & 3u)
         return STG_E_ALIGN;
-    if (a.flags & ~STG_PPO_CLIP_VF) return STG_E_ENUM;
-    stg::PolLaunch l;
-    if (int rc = stg::pol_configure(l)) return rc;
+    return STG_OK;
+}
+
+// the gradient kernel of K10 into d_work, then the fold of its grid partials in `kMode`
+template <PpoFold kMode>
+static int ppo_launch(const StgPpoArgs& a, double* raw, cudaStream_t s) {
+    PolLaunch l;
+    if (int rc = pol_configure(l)) return rc;
     const int grid = (int)STG_PPO_GRID(a.batch);
-    cudaStream_t s = (cudaStream_t)stream;
-    stg::policy_ppo_grad_kernel<<<grid, stg::kPolThreads, sizeof(stg::PpoShared), s>>>(a);
+    policy_ppo_grad_kernel<<<grid, kPolThreads, sizeof(PpoShared), s>>>(a);
     if (cudaError_t e = cudaGetLastError()) return (int)e;
-    stg::policy_ppo_fold_kernel<<<STG_POLICY_PARAMS / stg::kPolThreads + 1, stg::kPolThreads, 0, s>>>(a, grid);
+    policy_ppo_fold_kernel<kMode><<<STG_POLICY_PARAMS / kPolThreads + 1, kPolThreads, 0, s>>>(a, a.d_work, grid, raw);
+    return (int)cudaGetLastError();
+}
+
+}  // namespace stg
+
+extern "C" int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream) {
+    if (!args) return STG_E_NULL;
+    const StgPpoArgs& a = *args;
+    if (int rc = stg::ppo_check(a, true)) return rc;
+    if (a.flags & ~STG_PPO_CLIP_VF) return STG_E_ENUM;
+    return stg::ppo_launch<stg::kFoldScale>(a, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int stg_policy_ppo_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream) {
+    if (!args) return STG_E_NULL;
+    const StgPpoArgs& a = *args;
+    if (a.batch < 1) return STG_E_SIZE;
+    if (!d_sums) return STG_E_NULL;
+    if (int rc = stg::ppo_check(a, false)) return rc;
+    if ((uintptr_t)d_sums & 7u) return STG_E_ALIGN;
+    if (a.flags & ~STG_PPO_CLIP_VF) return STG_E_ENUM;
+    return stg::ppo_launch<stg::kFoldRaw>(a, d_sums, (cudaStream_t)stream);
+}
+
+extern "C" int stg_policy_ppo_finish_f32(const StgPpoArgs* args, const double* d_sums, int32_t ranks, void* stream) {
+    if (!args) return STG_E_NULL;
+    const StgPpoArgs& a = *args;
+    if (ranks < 1) return STG_E_SIZE;
+    if (!a.d_weights || !a.d_grad || !a.d_losses || !d_sums) return STG_E_NULL;
+    if ((uintptr_t)a.d_weights & 15u || (uintptr_t)d_sums & 7u || ((uintptr_t)a.d_grad | (uintptr_t)a.d_losses) & 3u)
+        return STG_E_ALIGN;
+    stg::policy_ppo_fold_kernel<stg::kFoldRanks><<<STG_POLICY_PARAMS / stg::kPolThreads + 1, stg::kPolThreads, 0,
+                                                   (cudaStream_t)stream>>>(a, d_sums, ranks, nullptr);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int stg_ppo_adv_moments_f64(const float* d_adv, int64_t n, double* d_out, void* stream) {
+    if (n < 0) return STG_E_SIZE;
+    if (!d_out || (n > 0 && !d_adv)) return STG_E_NULL;
+    if ((uintptr_t)d_adv & 3u || (uintptr_t)d_out & 7u) return STG_E_ALIGN;
+    stg::ppo_adv_moments_kernel<<<1, stg::kAdvThreads, 0, (cudaStream_t)stream>>>(d_adv, n, d_out);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int stg_ppo_adv_merge_f32(const double* d_moments, int32_t ranks, float* d_stats, void* stream) {
+    if (ranks < 1) return STG_E_SIZE;
+    if (!d_moments || !d_stats) return STG_E_NULL;
+    if ((uintptr_t)d_moments & 7u || (uintptr_t)d_stats & 3u) return STG_E_ALIGN;
+    stg::ppo_adv_merge_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d_moments, ranks, d_stats);
     return (int)cudaGetLastError();
 }

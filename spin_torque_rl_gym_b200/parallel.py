@@ -1,7 +1,8 @@
 """Multi-GPU plumbing: the env batch shards by contiguous global env-id ranges (one process per GPU, no data-path
 collective); one all-reduce(SUM) of the STG_NSTATS-element episode-statistics vector per rollout (SURVEY.md §8e — the
 reference analogue is the per-env EnvironmentMonitor, utils/monitoring.py:89-116), and, under a synchronised VecNormalize, one
-all-gather of the 27-double moment vector per env step (all_gather_moments)."""
+all-gather of the 27-double moment vector per env step (all_gather_moments), and, for data-parallel PPO, two all-gathers per
+minibatch (K12: the advantage moments and the gradient sums)."""
 from __future__ import annotations
 
 from typing import Dict, Tuple
@@ -76,8 +77,15 @@ def episode_metrics(totals: Dict[str, float]) -> Dict[str, float]:
     return out
 
 
+def world_size(group=None) -> int:
+    """The world size of the initialised process group, or 1 without one."""
+    import torch.distributed as dist
+    return dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+
+
 def all_gather_moments(local, group=None):
-    """[G, 27] stack of every rank's moment vector `local` [27] (float64, VecNormalize / K8), in rank order. The list form of
+    """[G, 27] stack of every rank's moment vector `local` [27] (float64, VecNormalize / K8), in rank order; any other 1-D
+    vector of the same size on every rank works too (the K12 advantage moments and PPO sums). The list form of
     all_gather, so it serves gloo (CPU tensors) and NCCL (CUDA tensors) alike; with NCCL it is enqueued on the current stream
     and nothing waits on the host. Without an initialised process group, or with world size 1, it returns `local[None]` and
     issues no collective."""

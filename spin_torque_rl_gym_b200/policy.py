@@ -304,7 +304,8 @@ class ActorCriticPolicy(nn.Module):
         return n, planes
 
     def ppo_backward(self, samples, clip_range: float = 0.2, clip_range_vf: Optional[float] = None,
-                     ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = True) -> PPOLosses:
+                     ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = True,
+                     data_parallel: bool = False) -> PPOLosses:
         """SB3's PPO.train() loss of one minibatch with the current weights, and the gradient of every parameter: the result
         of `optimizer.zero_grad(); loss.backward()`, in one launch of stg_policy_ppo_grad_f32 and its fold (K10).
 
@@ -318,32 +319,131 @@ class ActorCriticPolicy(nn.Module):
         are reassigned on every call, so `zero_grad(set_to_none=True)` between calls does no harm. Gradient clipping and the
         optimiser step are the caller's (`torch.nn.utils.clip_grad_norm_`, `torch.optim.Adam`). Returns PPOLosses; nothing
         is read back to the host, so early stopping on approx_kl costs the caller one synchronisation.
+
+        `data_parallel=True` (K12): under a process group of G ranks, `samples` is this rank's part of a global minibatch,
+        and every rank calls ppo_backward with a part of the same size. The loss and gradient are then those of the union of
+        the G parts, with the advantages normalised by the mean and std of the union (FP64 moments of each part, gathered and
+        merged in rank order), and are bit-identical on every rank: each rank computes the unscaled FP64 sums of its rows,
+        the G sums vectors (81.5 KB each) are all-gathered, and every rank folds them in rank order before the scaling. Two
+        all_gathers on the current stream, no host synchronisation. So any optimiser steps identically on every rank. Without
+        a process group, or with world size 1, the same kernels run without a collective.
         Raises StgError without CUDA, ValueError for an empty batch or planes of the wrong shape, dtype or device."""
+        if data_parallel:
+            return self._ppo_backward_ranks(samples, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage)
         n, planes = self._ppo_planes(samples)
         dev = self.log_std.device
         with _lib.device_guard(torch, dev):
-            w = self.pack_weights()
-            if self._grad is None or self._grad.device != dev:
-                self._grad = torch.empty(_lib.POLICY_PARAMS, dtype=torch.float32, device=dev)
             stats = None
             if normalize_advantage and n > 1:
                 adv = planes[4]
                 stats = torch.stack([adv.mean(), adv.std()])
             losses = torch.empty(_lib.PPO_LOSSES, dtype=torch.float32, device=dev)
             work = torch.empty(_lib.ppo_work_doubles(n), dtype=torch.float64, device=dev)
-            a = _lib.StgPpoArgs()
-            a.d_weights = w.data_ptr()
-            a.d_obs, a.d_action, a.d_old_value, a.d_old_log_prob, a.d_advantage, a.d_return = (t.data_ptr() for t in planes)
-            a.d_adv_stats = None if stats is None else stats.data_ptr()
-            a.d_grad, a.d_losses, a.d_work = self._grad.data_ptr(), losses.data_ptr(), work.data_ptr()
-            cr = float(clip_range)
-            a.clip_range, a.ratio_lo, a.ratio_hi = cr, 1.0 - cr, 1.0 + cr     # rounded to float32 as torch.clamp does
-            if clip_range_vf is not None:
-                a.flags = _lib.PPO_CLIP_VF
-                a.clip_range_vf = float(clip_range_vf)
-            a.ent_coef, a.vf_coef = float(ent_coef), float(vf_coef)
-            a.batch = n
+            a = self._ppo_args(n, planes, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
+            a.d_grad, a.d_losses, a.d_work = self._grad_buffer().data_ptr(), losses.data_ptr(), work.data_ptr()
             self._launch(_lib.load().stg_policy_ppo_grad_f32, a, "stg_policy_ppo_grad_f32")
+        self._set_grads()
+        return PPOLosses(*losses.unbind())
+
+    def _grad_buffer(self):
+        dev = self.log_std.device
+        if self._grad is None or self._grad.device != dev:
+            self._grad = torch.empty(_lib.POLICY_PARAMS, dtype=torch.float32, device=dev)
+        return self._grad
+
+    def _set_grads(self) -> None:
         for p, off in self._grad_slots():
             p.grad = self._grad[off:off + p.numel()].view_as(p)
+
+    def _ppo_args(self, n: int, planes, stats, clip_range, clip_range_vf, ent_coef, vf_coef) -> _lib.StgPpoArgs:
+        """K10's argument block for `planes` with the weights repacked; the outputs and d_work are the caller's."""
+        a = _lib.StgPpoArgs()
+        a.d_weights = self.pack_weights().data_ptr()
+        if planes is not None:
+            a.d_obs, a.d_action, a.d_old_value, a.d_old_log_prob, a.d_advantage, a.d_return = (t.data_ptr() for t in planes)
+        a.d_adv_stats = None if stats is None else stats.data_ptr()
+        cr = float(clip_range)
+        a.clip_range, a.ratio_lo, a.ratio_hi = cr, 1.0 - cr, 1.0 + cr     # rounded to float32 as torch.clamp does
+        if clip_range_vf is not None:
+            a.flags = _lib.PPO_CLIP_VF
+            a.clip_range_vf = float(clip_range_vf)
+        a.ent_coef, a.vf_coef = float(ent_coef), float(vf_coef)
+        a.batch = n
+        return a
+
+    # ---- K12 -----------------------------------------------------------------------------------------------------------------
+    def _ppo_backward_ranks(self, samples, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage) -> PPOLosses:
+        """ppo_backward(data_parallel=True): moments -> all_gather -> merge -> sums -> all_gather -> finish, on the current
+        stream of the policy's device."""
+        from .parallel import all_gather_moments, world_size
+        n, _ = self._ppo_planes(samples)
+        dev = self.log_std.device
+        with _lib.device_guard(torch, dev), torch.cuda.stream(torch.cuda.current_stream(dev)):
+            stats = None
+            if normalize_advantage and n * world_size() > 1:
+                stats = _adv_stats(all_gather_moments(_adv_moments(samples.advantages)))
+            sums = self._ppo_sums(samples, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
+            return self._ppo_finish(all_gather_moments(sums), ent_coef, vf_coef)
+
+    def _ppo_sums(self, samples, stats, clip_range: float = 0.2, clip_range_vf: Optional[float] = None,
+                  ent_coef: float = 0.0, vf_coef: float = 0.5):
+        """The unscaled FP64 sums of this part of a minibatch (stg_policy_ppo_sums_f32): a float64 [STG_PPO_PART] tensor.
+        `stats`: the float32 [2] (mean, std) to normalise the advantages with, or None."""
+        n, planes = self._ppo_planes(samples)
+        dev = self.log_std.device
+        with _lib.device_guard(torch, dev):
+            sums = torch.empty(_lib.PPO_PART, dtype=torch.float64, device=dev)
+            work = torch.empty(_lib.ppo_work_doubles(n), dtype=torch.float64, device=dev)
+            a = self._ppo_args(n, planes, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
+            a.d_work = work.data_ptr()
+            _lib.check(_lib.load().stg_policy_ppo_sums_f32(C.byref(a), sums.data_ptr(),
+                                                           torch.cuda.current_stream(dev).cuda_stream),
+                       "stg_policy_ppo_sums_f32")
+        return sums
+
+    def _ppo_finish(self, sums, ent_coef: float = 0.0, vf_coef: float = 0.5) -> PPOLosses:
+        """The loss and gradient of the union of the parts whose sums are the rows of `sums` (float64 [G, STG_PPO_PART], in
+        rank order), folded by stg_policy_ppo_finish_f32 into the policy's gradient buffer; sets every `.grad` to its view as
+        ppo_backward does."""
+        dev = self.log_std.device
+        sums = sums.reshape(-1, _lib.PPO_PART)
+        if sums.dtype != torch.float64 or sums.device != dev or sums.shape[0] < 1:
+            raise ValueError(f"sums must be a float64 [G, {_lib.PPO_PART}] tensor on {dev}")
+        sums = sums.contiguous()
+        with _lib.device_guard(torch, dev):
+            losses = torch.empty(_lib.PPO_LOSSES, dtype=torch.float32, device=dev)
+            a = self._ppo_args(0, None, None, 0.0, None, ent_coef, vf_coef)
+            a.d_grad, a.d_losses = self._grad_buffer().data_ptr(), losses.data_ptr()
+            _lib.check(_lib.load().stg_policy_ppo_finish_f32(C.byref(a), sums.data_ptr(), sums.shape[0],
+                                                             torch.cuda.current_stream(dev).cuda_stream),
+                       "stg_policy_ppo_finish_f32")
+        self._set_grads()
         return PPOLosses(*losses.unbind())
+
+
+def _adv_moments(adv):
+    """float64 [3] (n, mean, M2) of the float32 advantages `adv` [B] on the device (stg_ppo_adv_moments_f64)."""
+    adv = adv.reshape(-1)
+    if adv.dtype != torch.float32 or adv.device.type != "cuda":
+        raise ValueError("the advantages must be a float32 CUDA tensor")
+    adv = adv.contiguous()
+    out = torch.empty(_lib.PPO_ADV_MOMENTS, dtype=torch.float64, device=adv.device)
+    with _lib.device_guard(torch, adv.device):
+        _lib.check(_lib.load().stg_ppo_adv_moments_f64(adv.data_ptr(), adv.numel(), out.data_ptr(),
+                                                       torch.cuda.current_stream(adv.device).cuda_stream),
+                   "stg_ppo_adv_moments_f64")
+    return out
+
+
+def _adv_stats(moments):
+    """float32 [2] (mean, std with correction 1) of the union of the parts whose moments are the rows of `moments` (float64
+    [G, 3], in rank order): stg_ppo_adv_merge_f32, the d_adv_stats of K10."""
+    moments = moments.reshape(-1, _lib.PPO_ADV_MOMENTS).contiguous()
+    if moments.dtype != torch.float64 or moments.device.type != "cuda":
+        raise ValueError("the moments must be a float64 CUDA tensor")
+    out = torch.empty(2, dtype=torch.float32, device=moments.device)
+    with _lib.device_guard(torch, moments.device):
+        _lib.check(_lib.load().stg_ppo_adv_merge_f32(moments.data_ptr(), moments.shape[0], out.data_ptr(),
+                                                     torch.cuda.current_stream(moments.device).cuda_stream),
+                   "stg_ppo_adv_merge_f32")
+    return out

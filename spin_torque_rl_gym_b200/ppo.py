@@ -11,8 +11,8 @@ import torch
 from . import _lib
 from .envs import RolloutCollector
 from .optim import ClippedAdam
-from .parallel import all_reduce_stats, episode_metrics
-from .policy import ActorCriticPolicy
+from .parallel import all_gather_moments, all_reduce_stats, episode_metrics, world_size
+from .policy import ActorCriticPolicy, _adv_moments
 
 Schedule = Union[float, Callable[[float], float]]
 _LOG = _lib.ADAM_LOG_SLOTS
@@ -29,8 +29,8 @@ def _schedule(value: Optional[Schedule]) -> Optional[Callable[[float], float]]:
 class PPO:
     """`PPO(policy, env, learning_rate=3e-4, n_steps=2048, batch_size=64, n_epochs=10, gamma=0.99, gae_lambda=0.95,
     clip_range=0.2, clip_range_vf=None, normalize_advantage=True, ent_coef=0.0, vf_coef=0.5, max_grad_norm=0.5,
-    target_kl=None, seed=None, policy_kwargs=None)`: SB3's PPO signature and defaults for a SpinTorqueVectorEnv (or a
-    VecNormalize around one) with `autoreset=True`, on its device.
+    target_kl=None, seed=None, policy_kwargs=None, data_parallel=False)`: SB3's PPO signature and defaults for a
+    SpinTorqueVectorEnv (or a VecNormalize around one) with `autoreset=True`, on its device.
 
     `policy` is "MlpPolicy" (an `ActorCriticPolicy(env, seed=seed, **policy_kwargs)` built after `torch.manual_seed(seed)` when
     a seed is given) or an ActorCriticPolicy built for `env`. `self.rollout_buffer` is a `RolloutCollector(env, n_steps,
@@ -43,17 +43,32 @@ class PPO:
     appends to `self.log_history` a dict with SB3's logger keys (`train/...`); `learn()` adds `rollout/...` (of the rollout
     just collected, from the difference of the env's cumulative statistics) and `time/...` to it.
 
+    `data_parallel=True` trains one policy over the G ranks of a process group (K12), each rank holding its shard of the
+    envs (`parallel.shard_range`, the same `num_envs` on every rank). `batch_size` and `num_timesteps` are global: each
+    minibatch is the union of one local minibatch of `batch_size // G` rows per rank, normalised with the advantage statistics
+    of that union, and `ppo_backward(data_parallel=True)` gives every rank the same gradient and losses, so the weights, the
+    `target_kl` gate and `log_history` are bit-identical on every rank after every step. The constructor broadcasts rank 0's
+    parameters and optimiser state and checks that every rank has the same `num_envs`, `batch_size` and policy seed; the
+    policy seed keys the action noise by global env id, so the rollout of G ranks is that of one process over all the envs.
+    `explained_variance` comes from FP64 moments gathered across the ranks. Per minibatch that costs two all_gathers on the
+    current stream (3 and 10,192 doubles per rank). Without a process group, or with world size 1, it runs the same kernels
+    with no collective.
+
     Raises ValueError for `batch_size < 2` with `normalize_advantage` (SB3 asserts it), a policy of another kind, or an env the
-    collector rejects; NotImplementedError under a process group of world size > 1 (each rank would train its own policy)."""
+    collector rejects, and with `data_parallel=True` for a `batch_size` that G does not divide, a VecNormalize that does not
+    share its statistics across the ranks, or ranks that disagree; NotImplementedError under a process group of world size
+    > 1 without `data_parallel=True` (each rank would train its own policy)."""
 
     def __init__(self, policy: Union[str, ActorCriticPolicy], env, learning_rate: Schedule = 3e-4, n_steps: int = 2048,
                  batch_size: int = 64, n_epochs: int = 10, gamma: float = 0.99, gae_lambda: float = 0.95,
                  clip_range: Schedule = 0.2, clip_range_vf: Optional[Schedule] = None, normalize_advantage: bool = True,
                  ent_coef: float = 0.0, vf_coef: float = 0.5, max_grad_norm: Optional[float] = 0.5,
-                 target_kl: Optional[float] = None, seed: Optional[int] = None, policy_kwargs: Optional[Dict[str, Any]] = None):
-        import torch.distributed as dist
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-            raise NotImplementedError("PPO trains on one rank; data-parallel training across ranks is not implemented")
+                 target_kl: Optional[float] = None, seed: Optional[int] = None, policy_kwargs: Optional[Dict[str, Any]] = None,
+                 data_parallel: bool = False):
+        ranks = world_size()
+        if ranks > 1 and not data_parallel:
+            raise NotImplementedError("PPO(data_parallel=False) trains on one rank; under a process group of world size "
+                                      f"{ranks} pass data_parallel=True to train one policy across the ranks")
         if n_steps < 1 or n_epochs < 1 or batch_size < 1:
             raise ValueError(f"n_steps, n_epochs and batch_size must be positive, got {n_steps}, {n_epochs}, {batch_size}")
         if normalize_advantage and batch_size < 2:
@@ -71,6 +86,9 @@ class PPO:
             raise ValueError("policy_kwargs apply to 'MlpPolicy' only")
         elif policy.num_envs != env.num_envs or policy.log_std.device != torch.device(env.device):
             raise ValueError("the policy was built for another env (device or num_envs differ)")
+        if data_parallel:
+            _check_data_parallel(env, batch_size, ranks)
+        self.data_parallel, self.ranks = bool(data_parallel), ranks if data_parallel else 1
         self.env, self.policy = env, policy
         self.n_steps, self.batch_size, self.n_epochs = int(n_steps), int(batch_size), int(n_epochs)
         self.gamma, self.gae_lambda = gamma, gae_lambda
@@ -87,8 +105,25 @@ class PPO:
         self._n_updates = 0
         self._total_timesteps = 0
         self._current_progress_remaining = 1.0
+        if self.ranks > 1:
+            self._synchronise_ranks()
         self._last_stats = all_reduce_stats(env.stats_tensor())
         self.log_history: List[Dict[str, float]] = []
+
+    def _synchronise_ranks(self) -> None:
+        """Data-parallel start-up: check that the ranks agree on num_envs, batch_size and the policy seed, then broadcast
+        rank 0's parameters and optimiser state."""
+        import torch.distributed as dist
+        pol, opt = self.policy, self.policy.optimizer
+        seed = pol.seed - (1 << 64) if pol.seed >= 1 << 63 else pol.seed          # the 64-bit seed as an int64
+        mine = torch.tensor([self.env.num_envs, self.batch_size, seed], dtype=torch.int64, device=pol.log_std.device)
+        every = all_gather_moments(mine).cpu()
+        if not bool((every == every[0]).all()):
+            raise ValueError("data-parallel PPO needs the same num_envs, batch_size and policy seed on every rank, got "
+                             f"{every.tolist()} (rows: ranks)")
+        with torch.no_grad():
+            for t in [p.data for p in pol.parameters()] + [opt._exp_avg, opt._exp_avg_sq, opt._step_count]:
+                dist.broadcast(t, src=0)
 
     def learn(self, total_timesteps: int, reset_num_timesteps: bool = True) -> "PPO":
         """SB3's learn(): until num_timesteps reaches total_timesteps, collect n_steps x num_envs samples on the fused path,
@@ -103,7 +138,7 @@ class PPO:
         col = self.rollout_buffer
         while self.num_timesteps < total_timesteps:
             stats = col.collect(self.policy)
-            self.num_timesteps += self.n_steps * self.env.num_envs
+            self.num_timesteps += self.n_steps * self.env.num_envs * self.ranks
             iteration += 1
             self._current_progress_remaining = 1.0 - float(self.num_timesteps) / float(total_timesteps)
             col.compute_returns_and_advantage(self.gamma, self.gae_lambda)
@@ -117,8 +152,9 @@ class PPO:
         return self
 
     def train(self) -> Dict[str, float]:
-        """SB3's train() over the collected rollout: n_epochs epochs of get(batch_size) minibatches, each one ppo_backward
-        launch and one ClippedAdam launch that logs its losses and applies the gate. Returns the logged dict."""
+        """SB3's train() over the collected rollout: n_epochs epochs of get(batch_size) minibatches (get(batch_size // G)
+        per rank with data_parallel), each one ppo_backward launch and one ClippedAdam launch that logs its losses and applies
+        the gate. Returns the logged dict."""
         pol, opt, col = self.policy, self.policy.optimizer, self.rollout_buffer
         progress = self._current_progress_remaining
         lr = float(self.lr_schedule(progress))
@@ -131,17 +167,21 @@ class PPO:
         gate.fill_(1)
         for _ in range(self.n_epochs):
             log[_LOG["EPOCH_KL"]:_LOG["EPOCH_COUNT"] + 1].zero_()
-            for batch in col.get(self.batch_size):
+            for batch in col.get(self.batch_size // self.ranks):
                 losses = pol.ppo_backward(batch, clip_range, clip_range_vf, self.ent_coef, self.vf_coef,
-                                          self.normalize_advantage)
+                                          self.normalize_advantage, data_parallel=self.data_parallel)
                 opt._step(losses, gate, log, self.target_kl)
             self._n_updates += 1
             if self.target_kl is not None and int(gate.item()) == 0:
                 break
         with torch.no_grad():
             values, returns = col.values.reshape(-1), col.returns.reshape(-1)
-            var_y = returns.var(correction=0)
-            explained_var = torch.where(var_y == 0, math.nan, 1 - (returns - values).var(correction=0) / var_y)
+            if self.data_parallel:
+                moments = all_gather_moments(torch.cat([_adv_moments(returns), _adv_moments(returns - values)]))
+                explained_var = _explained_variance(moments.reshape(-1, 2, _lib.PPO_ADV_MOMENTS))
+            else:
+                var_y = returns.var(correction=0)
+                explained_var = torch.where(var_y == 0, math.nan, 1 - (returns - values).var(correction=0) / var_y)
             count = log[_LOG["COUNT"]]
             row = torch.stack([log[_LOG["ENTROPY"]] / count, log[_LOG["PG"]] / count, log[_LOG["VALUE"]] / count,
                                log[_LOG["EPOCH_KL"]] / log[_LOG["EPOCH_COUNT"]], log[_LOG["CLIP"]] / count,
@@ -161,3 +201,22 @@ class PPO:
     def predict(self, obs, deterministic: bool = False):
         """The policy's predict: (env actions, None)."""
         return self.policy.predict(obs, deterministic=deterministic)
+
+
+def _check_data_parallel(env, batch_size: int, ranks: int) -> None:
+    """The ValueErrors of PPO(data_parallel=True) that need no collective."""
+    from .envs.vec_normalize import VecNormalize
+    if batch_size % ranks:
+        raise ValueError(f"data-parallel PPO needs batch_size divisible by the world size {ranks}, got {batch_size}")
+    if isinstance(env, VecNormalize) and not env._syncing():
+        raise ValueError("data-parallel PPO needs a VecNormalize that shares its statistics across the ranks (sync=None or "
+                         "True), or the ranks would normalise their observations differently")
+
+
+def _explained_variance(moments):
+    """1 - Var(returns - values) / Var(returns) (population variances, NaN when Var(returns) is 0) from moments [G, 2, 3]:
+    per rank the FP64 (n, mean, M2) of the returns and of returns - values. Each is folded in rank order with K12's merge
+    (stg_ppo_adv_merge_f32 gives torch's std with correction 1, whose square ratio is the ratio of the M2)."""
+    from .policy import _adv_stats
+    std_y, std_d = _adv_stats(moments[:, 0])[1].double(), _adv_stats(moments[:, 1])[1].double()
+    return torch.where(std_y == 0, math.nan, 1 - (std_d * std_d) / (std_y * std_y))
