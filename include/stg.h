@@ -929,6 +929,62 @@ typedef struct StgAdamArgs {
 } StgAdamArgs;
 int stg_policy_adam_f32(const StgAdamArgs* args, void* stream);
 
+/* ---- K10, A2C instance: A2C loss and gradient of the ActorCriticPolicy (Stable-Baselines3's A2C.train() step) -----------
+ * The K10 kernel and fold with the policy head replaced: for B rows (in A2C one update covers the whole rollout, n_steps * N
+ * rows), the loss of SB3's A2C.train() and its gradient with respect to every parameter. Per row i, in FP32, the forward pass
+ * and A_i are K10's (A_i normalised with d_adv_stats, or the raw advantage when it is NULL); then
+ *   pg_i = A_i * logp_i (one rounding);  vpred_i = values_i (no value clip).
+ * Losses (d_losses, STG_PPO_LOSSES floats; sums over rows in FP64, the rest in FP64 and rounded once):
+ *   [0] loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss   [1] policy_loss = -sum(pg) / B
+ *   [2] value_loss = sum((return - values)^2) / B (F.mse_loss)   [3] entropy_loss as K10   [4] 0   [5] 0
+ * Gradient: d(-pg_i)/d logp_i = -A_i, then K10's backward pass, tiling, FP64 partials, fold and scaling (1/B for the actor,
+ * 2 vf_coef/B for the critic, -ent_coef added to each log_std). In d_work the pmin slot of a partial holds sum(pg) and the kl
+ * and clipped slots stay 0. Determinism as K10: the bits depend only on B, the weights and the data.
+ *   stg_policy_a2c_grad_f32   d_grad and d_losses as above; d_work holds STG_PPO_WORK_DOUBLES(B) doubles, and the grid is
+ *                             STG_PPO_GRID(B) CTAs, as for K10.
+ *   stg_policy_a2c_sums_f32   the unscaled FP64 sums for K12 in the STG_PPO_PART layout (stg_policy_ppo_sums_f32's layout: the
+ *                             gradient sums, sum(pg) at STG_PPO_PART_LOSS, the squared error sum next, 0 in the kl and
+ *                             clipped slots, the row count at STG_PPO_PART_COUNT). stg_policy_ppo_finish_f32 folds them in
+ *                             rank order into the A2C losses and gradient of the union; slots [4] and [5] come out 0.
+ * What differs from K10's arguments: d_old_value and d_old_log_prob are not read and may be NULL (they are not checked for
+ * alignment either); clip_range, ratio_lo, ratio_hi and clip_range_vf are not read; any nonzero flags, STG_PPO_CLIP_VF
+ * included, -> STG_E_ENUM (A2C has no value clip).
+ * Errors, in this order:
+ *   grad: args NULL -> STG_E_NULL; batch < 1 -> STG_E_SIZE; d_weights, d_obs, d_action, d_advantage, d_return, d_grad,
+ *         d_losses or d_work NULL -> STG_E_NULL; K10's alignments without the old planes -> STG_E_ALIGN; flags != 0 ->
+ *         STG_E_ENUM.
+ *   sums: args NULL -> STG_E_NULL; batch < 1 -> STG_E_SIZE; d_sums NULL, or a pointer the grad entry needs other than d_grad
+ *         and d_losses NULL -> STG_E_NULL; those alignments, d_sums not 8-B aligned -> STG_E_ALIGN; flags != 0 ->
+ *         STG_E_ENUM. */
+int stg_policy_a2c_grad_f32(const StgPpoArgs* args, void* stream);
+int stg_policy_a2c_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream);
+
+/* ---- K13: clipped RMSprop step of the ActorCriticPolicy (clip_grad_norm_ + torch.optim.RMSprop, SB3's A2C optimiser) -----
+ * One launch of one CTA of STG_ADAM_THREADS threads over the STG_POLICY_PARAMS parameters in the K10 gradient layout:
+ * 1. *d_step += 1.0f (float32): torch's per-parameter `step` state. The update does not read it.
+ * 2. Clip (STG_RMSPROP_CLIP): K11's step 2 exactly (the same FP64 chains and tree, clip_coef, and the clipped gradient written
+ *    back to d_grad).
+ * 3. RMSprop: torch.optim.RMSprop's single-tensor update with momentum 0, centered=False, no weight decay, not maximize. The
+ *    scalars are rounded to float32 once: alpha_f = float32(alpha), w = float32(1 - alpha), eps_f = float32(eps),
+ *    lr_f = float32(lr). Per element, in float32 with every operation IEEE-rounded on its own (no contraction):
+ *      sq = sq * alpha_f + (w * g) * g                                 (mul_, then addcmul_ with value = 1 - alpha)
+ *      avg = sqrt(sq) + eps_f                                          (sqrt, then add_(eps))
+ *      p = p - (lr_f * g) / avg                                        (addcdiv_ with value = -lr, K11's order)
+ *    with g the clipped gradient; parameters are addressed through d_param as in K11.
+ * Errors, in this order: args NULL, a d_param, d_grad, d_square_avg or d_step pointer NULL -> STG_E_NULL; any of them not 4-B
+ * aligned -> STG_E_ALIGN; flags other than STG_RMSPROP_CLIP -> STG_E_ENUM. */
+#define STG_RMSPROP_CLIP 0x1u      /* clip the global L2 norm to max_grad_norm                        */
+typedef struct StgRmspropArgs {
+    float* d_param[STG_ADAM_TENSORS];  /* each parameter's own contiguous storage (the nn.Parameter data) */
+    float* d_grad;                     /* [STG_POLICY_PARAMS] K10 layout; clipped in place, as clip_grad_norm_ does */
+    float* d_square_avg;               /* [STG_POLICY_PARAMS] */
+    float* d_step;                     /* [1] RMSprop's step count, float32 as torch keeps it */
+    double lr, alpha, eps, max_grad_norm;
+    uint32_t flags;                    /* STG_RMSPROP_CLIP */
+    uint32_t reserved;
+} StgRmspropArgs;
+int stg_policy_rmsprop_f32(const StgRmspropArgs* args, void* stream);
+
 /* FMA-pipe throughput probe (bench.py's measured FP32/FP64 roofline denominator): blocks*256 threads x iters*64 FMAs.
  * f64 = 0: FFMA, 1: DFMA, 2: packed FFMA2 (iters*64 instructions = iters*128 FMAs per thread).
  * d_out: >= blocks*256 elements of the probed type (8 bytes each for modes 1, 2; never written in practice). */

@@ -14,8 +14,9 @@ from . import _lib, build, params  # noqa: F401
 from .envs import (RolloutCollector, SB3VecEnvAdapter, SpinTorqueArrayEnv, SpinTorqueArrayVectorEnv,  # noqa: F401
                    SpinTorqueEnv, SpinTorqueVectorEnv, VecNormalize, make, register_with_gymnasium)
 from .parallel import all_gather_moments, all_reduce_stats, shard_range  # noqa: F401
-from .policy import ActorCriticPolicy, PPOLosses  # noqa: F401
-from .optim import ClippedAdam  # noqa: F401
+from .policy import A2CLosses, ActorCriticPolicy, PPOLosses  # noqa: F401
+from .optim import ClippedAdam, ClippedRMSprop  # noqa: F401
 from .ppo import PPO  # noqa: F401
+from .a2c import A2C  # noqa: F401
 
 register_with_gymnasium()

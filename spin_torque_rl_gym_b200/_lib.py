@@ -61,6 +61,8 @@ ADAM_TENSORS = 13
 ADAM_LOG = 8
 ADAM_LOG_SLOTS = {"PG": 0, "VALUE": 1, "ENTROPY": 2, "CLIP": 3, "COUNT": 4, "EPOCH_KL": 5, "EPOCH_COUNT": 6, "LAST_LOSS": 7}
 ADAM_CLIP, ADAM_TARGET_KL = 0x1, 0x2
+# K13 clipped RMSprop (include/stg.h STG_RMSPROP_*)
+RMSPROP_CLIP = 0x1
 
 
 def ppo_grid(batch: int) -> int:
@@ -233,6 +235,12 @@ class StgAdamArgs(C.Structure):
                 ("max_grad_norm", C.c_double), ("target_kl", C.c_double), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+class StgRmspropArgs(C.Structure):
+    _fields_ = [("d_param", C.c_void_p * ADAM_TENSORS), ("d_grad", C.c_void_p), ("d_square_avg", C.c_void_p),
+                ("d_step", C.c_void_p), ("lr", C.c_double), ("alpha", C.c_double), ("eps", C.c_double),
+                ("max_grad_norm", C.c_double), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
+
+
 class StgEnergyParams(C.Structure):
     _fields_ = [("mu0", C.c_double), ("saturation_magnetization", C.c_double), ("volume", C.c_double),
                 ("uniaxial_anisotropy", C.c_double), ("easy_axis", c_double3), ("demag_factors", c_double3)]
@@ -290,6 +298,9 @@ SYMBOLS = {
     "stg_ppo_adv_moments_f64": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "stg_ppo_adv_merge_f32": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "stg_policy_adam_f32": (C.c_int, [C.POINTER(StgAdamArgs), C.c_void_p]),
+    "stg_policy_a2c_grad_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p]),
+    "stg_policy_a2c_sums_f32": (C.c_int, [C.POINTER(StgPpoArgs), C.c_void_p, C.c_void_p]),
+    "stg_policy_rmsprop_f32": (C.c_int, [C.POINTER(StgRmspropArgs), C.c_void_p]),
     "stg_probe_fma": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

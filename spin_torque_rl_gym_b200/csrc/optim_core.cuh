@@ -1,5 +1,6 @@
-// optim_core.cuh — arithmetic of K11, the clipped Adam step (include/stg.h, stg_policy_adam_f32), shared by optim_kernels.cu and
-// the host build in tests/test_ppo_train.py.
+// optim_core.cuh — arithmetic of K11, the clipped Adam step (include/stg.h, stg_policy_adam_f32), and of K13, the clipped
+// RMSprop step (stg_policy_rmsprop_f32), shared by optim_kernels.cu and the host builds in tests/test_ppo_train.py and
+// tests/test_a2c.py.
 //
 // Specification: torch.nn.utils.clip_grad_norm_ followed by torch.optim.Adam's single-tensor update (foreach=False,
 // capturable=False, no weight decay, no amsgrad), in torch's order of operations. Every float32 product, sum, quotient and
@@ -110,6 +111,29 @@ STG_HD float adam_element(float p, float g, float& m, float& v, const AdamCoef& 
     v = Pk<float>::add(Pk<float>::mul(v, c.b2), Pk<float>::mul(Pk<float>::mul(c.w2, g), g));
     const float denom = Pk<float>::add(adam_div(adam_sqrt(v), c.bc2_sqrt), c.eps);
     return adam_sub(p, adam_div(Pk<float>::mul(c.step_size, m), denom));
+}
+
+// ---- K13: torch.optim.RMSprop's single-tensor update (momentum 0, centered=False, no weight decay, not maximize) ---------
+
+// the float32 scalars of one RMSprop step
+struct RmspropCoef {
+    float alpha, w, eps, lr;
+};
+
+STG_HD RmspropCoef rmsprop_coef(double lr, double alpha, double eps) {
+    RmspropCoef c;
+    c.alpha = (float)alpha;
+    c.w = (float)(1.0 - alpha);
+    c.eps = (float)eps;
+    c.lr = (float)lr;
+    return c;
+}
+
+// one element: the running square average sq is updated in place and the new parameter is returned
+STG_HD float rmsprop_element(float p, float g, float& sq, const RmspropCoef& c) {
+    sq = Pk<float>::add(Pk<float>::mul(sq, c.alpha), Pk<float>::mul(Pk<float>::mul(c.w, g), g));   // mul_, addcmul_
+    const float avg = Pk<float>::add(adam_sqrt(sq), c.eps);                                          // sqrt, add_(eps)
+    return adam_sub(p, adam_div(Pk<float>::mul(c.lr, g), avg));                                      // addcdiv_(value=-lr)
 }
 
 }  // namespace stg

@@ -147,6 +147,23 @@ STG_HD float pol_ppo_policy_row(float logp, float old_logp, float adv, const Pol
     return K::mul(-dmin, r);                                              // exp's backward: times its result
 }
 
+// The policy part of an A2C row (SB3's A2C.train(): policy_loss = -(A * logp).mean()): adds A * logp to sums[kPpoPmin], so
+// that the fold's -sum / B is A2C's policy loss, and returns d(-A logp)/d logp. The kl and clipped sums stay 0.
+STG_HD float pol_a2c_policy_row(float logp, float adv, double* sums) {
+    sums[kPpoPmin] += (double)Pk<float>::mul(adv, logp);
+    return -adv;
+}
+
+// the loss a K10 instance computes: SB3's PPO (clipped surrogate, optional value clip) or A2C (plain policy gradient,
+// unclipped value MSE; old values and old log-probabilities are not read)
+enum PolLoss { kLossPpo = 0, kLossA2c = 1 };
+
+// the policy part of a row under loss L: d(policy loss term)/d logp
+template <PolLoss L>
+STG_HD float pol_policy_row(float logp, float old_logp, float adv, const PolPpoCoef& c, double* sums) {
+    return L == kLossA2c ? pol_a2c_policy_row(logp, adv, sums) : pol_ppo_policy_row(logp, old_logp, adv, c, sums);
+}
+
 // Normal.log_prob's backward for a row with d(.)/d logp = gl and scale = STD: d/d mean_d and d/d log_std_d
 STG_HD void pol_ppo_gauss_row(float gl, const float act[2], const float mean[2], const float* w, float gm[2], float gs[2]) {
     using K = Pk<float>;
@@ -220,7 +237,9 @@ STG_HD void pol_adv_stats(const double* moments, int ranks, float out[2]) {
 
 // One row's forward pass (K9's chains) and backward pass on the host: adds its unscaled gradient to grad (the d_grad layout)
 // and its loss sums to sums. `adv` is already normalised. The kernel computes the same per-row quantities, tiled; its
-// weight-gradient sums run over the rows of a tile in FP32 instead of one product per row.
+// weight-gradient sums run over the rows of a tile in FP32 instead of one product per row. With L = kLossA2c, old_value and
+// old_logp are not read and c.clip_value must be false.
+template <PolLoss L = kLossPpo>
 STG_HD void pol_backward_row(const float* w, const float* obs, const float act[2], float old_value, float old_logp, float adv,
                              float ret, const PolPpoCoef& c, double* grad, double* sums) {
     float h1[kPolHidden], h2[kPolHidden], d2[kPolHidden];
@@ -244,7 +263,7 @@ STG_HD void pol_backward_row(const float* w, const float* obs, const float act[2
                 const float t = pol_log_prob_term(act[d], mean[d], w[STG_POLICY_STD + d], w[STG_POLICY_LOG_SCALE + d]);
                 logp = d == 0 ? t : Pk<float>::add(logp, t);
             }
-            const float gl = pol_ppo_policy_row(logp, old_logp, adv, c, sums);
+            const float gl = pol_policy_row<L>(logp, old_logp, adv, c, sums);
             pol_ppo_gauss_row(gl, act, mean, w, gm, gs);
             for (int k = 0; k < kPolHidden; ++k) {
                 grad[STG_POLICY_ACT_W + k] += (double)h2[k] * gm[0];

@@ -206,7 +206,7 @@ __global__ void __launch_bounds__(kPolThreads, 2) policy_value_kernel(const StgP
     if (queued > 0) pol_value_tile(s, a, queued);
 }
 
-// ---- K10: PPO loss and gradient (stg_policy_ppo_grad_f32) ----------------------------------------------------------------
+// ---- K10: PPO and A2C loss and gradient (stg_policy_ppo_grad_f32, stg_policy_a2c_grad_f32) -------------------------------
 // A grid of STG_PPO_GRID(B) persistent CTAs walks tiles of kPolTile rows (CTA b: tiles b, b + grid, ...). Per tile and network
 // (the critic, then the actor, so that only one network's activations are held):
 //   forward   pol_layer twice: h1 into plane a, h2 into plane h (K9's chains and bits);
@@ -224,7 +224,8 @@ __global__ void __launch_bounds__(kPolThreads, 2) policy_value_kernel(const StgP
 // in FP64 to its CTA's partial in d_work (always the same thread for the same element, so no atomics). The per-row sums (loss
 // terms, log_std) are FP64 in the row's thread and reduced in thread order at the end. ppo_fold_kernel then sums the partials
 // in CTA order. Shared memory: 40.75 KB of weights, x, two 64-row planes and two 128-row gradient channels, 113.0 KB, so two
-// CTAs fit on an SM.
+// CTAs fit on an SM. The loss is a template parameter: the A2C instance takes pol_a2c_policy_row as its policy head, has no
+// value clip and reads neither old plane; the tiling, the backward pass and the fold are the same code.
 constexpr int kPpoSums = 6;                             // per-row FP64 sums: the four loss sums and d/d log_std
 static_assert(STG_PPO_TILE == kPolTile && kPolThreads == 256, "stg.h and the K10 tiling disagree");
 
@@ -388,13 +389,15 @@ __device__ __forceinline__ void ppo_dw1(const PpoShared& s, int gw1, int gb1, do
     if (kq == 0) ppo_add(part, gb1 + o, db, first);
 }
 
+template <PolLoss kLoss>
 __global__ void __launch_bounds__(kPolThreads, 2) policy_ppo_grad_kernel(const StgPpoArgs a) {
     extern __shared__ __align__(16) unsigned char pol_smem[];
     PpoShared& s = *reinterpret_cast<PpoShared*>(pol_smem);
     pol_load_weights(s.w, a.d_weights);
     const int64_t n = a.batch, tiles = (n + kPolTile - 1) / kPolTile;
     const int e = threadIdx.x;
-    const PolPpoCoef c{a.clip_range, a.ratio_lo, a.ratio_hi, a.clip_range_vf, (a.flags & STG_PPO_CLIP_VF) != 0u};
+    const PolPpoCoef c{a.clip_range, a.ratio_lo, a.ratio_hi, a.clip_range_vf,
+                       kLoss == kLossPpo && (a.flags & STG_PPO_CLIP_VF) != 0u};
     float stats[2] = {0.0f, 0.0f};
     if (a.d_adv_stats) stats[0] = __ldg(a.d_adv_stats), stats[1] = __ldg(a.d_adv_stats + 1);
     double* part = a.d_work + (int64_t)blockIdx.x * STG_PPO_PART;
@@ -413,7 +416,10 @@ __global__ void __launch_bounds__(kPolThreads, 2) policy_ppo_grad_kernel(const S
         if (e < kPolTile) {
             const float v = pol_head(s.w, s.h, e, STG_POLICY_VAL_W, 1, 0, s.w[STG_POLICY_VAL_B]);
             float gv = 0.0f;
-            if (e < count) gv = pol_ppo_value_row(v, __ldg(a.d_old_value + base + e), __ldg(a.d_return + base + e), c, sums);
+            if (e < count) {
+                const float old_v = kLoss == kLossPpo ? __ldg(a.d_old_value + base + e) : 0.0f;
+                gv = pol_ppo_value_row(v, old_v, __ldg(a.d_return + base + e), c, sums);
+            }
             s.g[0][e] = gv;
         }
         __syncthreads();
@@ -439,7 +445,8 @@ __global__ void __launch_bounds__(kPolThreads, 2) policy_ppo_grad_kernel(const S
                     lp = d == 0 ? t : Pk<float>::add(lp, t);
                 }
                 const float adv = pol_ppo_advantage(__ldg(a.d_advantage + i), a.d_adv_stats ? stats : nullptr);
-                const float gl = pol_ppo_policy_row(lp, __ldg(a.d_old_log_prob + i), adv, c, sums);
+                const float old_lp = kLoss == kLossPpo ? __ldg(a.d_old_log_prob + i) : 0.0f;
+                const float gl = pol_policy_row<kLoss>(lp, old_lp, adv, c, sums);
                 pol_ppo_gauss_row(gl, act, mean, s.w, gm, gs);
                 sums[4] += (double)gs[0];
                 sums[5] += (double)gs[1];
@@ -560,7 +567,9 @@ static int pol_configure(PolLaunch& out) {
     PolLaunch l;
     if ((e = cudaFuncSetAttribute(policy_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(policy_value_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(policy_ppo_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        (e = cudaFuncSetAttribute(policy_ppo_grad_kernel<kLossPpo>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)sizeof(PpoShared))) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(policy_ppo_grad_kernel<kLossA2c>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)sizeof(PpoShared))) != cudaSuccess ||
         (e = cudaDeviceGetAttribute(&l.sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess ||
         (e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&l.per_sm, policy_act_kernel, kPolThreads, smem)) != cudaSuccess)
@@ -613,27 +622,37 @@ extern "C" int stg_policy_value_f32(const StgPolicyArgs* args, void* stream) {
 
 namespace stg {
 
-// K10's argument checks, with the gradient and loss outputs required or not (K12's sums)
+// K10's argument checks, with the gradient and loss outputs required or not (K12's sums); the A2C instance reads neither old
+// plane, so under kLossA2c they may be NULL and are not checked
+template <PolLoss kLoss>
 static int ppo_check(const StgPpoArgs& a, bool outputs) {
+    const bool old = kLoss == kLossPpo;
     if (a.batch < 1) return STG_E_SIZE;
-    if (!a.d_weights || !a.d_obs || !a.d_action || !a.d_old_value || !a.d_old_log_prob || !a.d_advantage || !a.d_return ||
-        (outputs && (!a.d_grad || !a.d_losses)) || !a.d_work)
+    if (!a.d_weights || !a.d_obs || !a.d_action || (old && (!a.d_old_value || !a.d_old_log_prob)) || !a.d_advantage ||
+        !a.d_return || (outputs && (!a.d_grad || !a.d_losses)) || !a.d_work)
         return STG_E_NULL;
     if (((uintptr_t)a.d_weights | (uintptr_t)a.d_obs) & 15u) return STG_E_ALIGN;
     if (((uintptr_t)a.d_action | (uintptr_t)a.d_work) & 7u) return STG_E_ALIGN;
-    if (((uintptr_t)a.d_old_value | (uintptr_t)a.d_old_log_prob | (uintptr_t)a.d_advantage | (uintptr_t)a.d_return |
-         (uintptr_t)a.d_adv_stats | (uintptr_t)a.d_grad | (uintptr_t)a.d_losses) & 3u)
+    const uintptr_t old_planes = old ? ((uintptr_t)a.d_old_value | (uintptr_t)a.d_old_log_prob) : 0u;
+    if ((old_planes | (uintptr_t)a.d_advantage | (uintptr_t)a.d_return | (uintptr_t)a.d_adv_stats | (uintptr_t)a.d_grad |
+         (uintptr_t)a.d_losses) & 3u)
         return STG_E_ALIGN;
     return STG_OK;
 }
 
-// the gradient kernel of K10 into d_work, then the fold of its grid partials in `kMode`
-template <PpoFold kMode>
+// flags K10 accepts under kLoss: STG_PPO_CLIP_VF for PPO, none for A2C (it has no value clip)
+template <PolLoss kLoss>
+static int ppo_check_flags(const StgPpoArgs& a) {
+    return a.flags & ~(kLoss == kLossPpo ? STG_PPO_CLIP_VF : 0u) ? STG_E_ENUM : STG_OK;
+}
+
+// the gradient kernel of K10 under kLoss into d_work, then the fold of its grid partials in `kMode`
+template <PolLoss kLoss, PpoFold kMode>
 static int ppo_launch(const StgPpoArgs& a, double* raw, cudaStream_t s) {
     PolLaunch l;
     if (int rc = pol_configure(l)) return rc;
     const int grid = (int)STG_PPO_GRID(a.batch);
-    policy_ppo_grad_kernel<<<grid, kPolThreads, sizeof(PpoShared), s>>>(a);
+    policy_ppo_grad_kernel<kLoss><<<grid, kPolThreads, sizeof(PpoShared), s>>>(a);
     if (cudaError_t e = cudaGetLastError()) return (int)e;
     policy_ppo_fold_kernel<kMode><<<STG_POLICY_PARAMS / kPolThreads + 1, kPolThreads, 0, s>>>(a, a.d_work, grid, raw);
     return (int)cudaGetLastError();
@@ -641,23 +660,47 @@ static int ppo_launch(const StgPpoArgs& a, double* raw, cudaStream_t s) {
 
 }  // namespace stg
 
-extern "C" int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream) {
+namespace stg {
+
+// stg_policy_{ppo,a2c}_grad_f32
+template <PolLoss kLoss>
+static int ppo_grad_entry(const StgPpoArgs* args, void* stream) {
     if (!args) return STG_E_NULL;
     const StgPpoArgs& a = *args;
-    if (int rc = stg::ppo_check(a, true)) return rc;
-    if (a.flags & ~STG_PPO_CLIP_VF) return STG_E_ENUM;
-    return stg::ppo_launch<stg::kFoldScale>(a, nullptr, (cudaStream_t)stream);
+    if (int rc = ppo_check<kLoss>(a, true)) return rc;
+    if (int rc = ppo_check_flags<kLoss>(a)) return rc;
+    return ppo_launch<kLoss, kFoldScale>(a, nullptr, (cudaStream_t)stream);
 }
 
-extern "C" int stg_policy_ppo_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream) {
+// stg_policy_{ppo,a2c}_sums_f32
+template <PolLoss kLoss>
+static int ppo_sums_entry(const StgPpoArgs* args, double* d_sums, void* stream) {
     if (!args) return STG_E_NULL;
     const StgPpoArgs& a = *args;
     if (a.batch < 1) return STG_E_SIZE;
     if (!d_sums) return STG_E_NULL;
-    if (int rc = stg::ppo_check(a, false)) return rc;
+    if (int rc = ppo_check<kLoss>(a, false)) return rc;
     if ((uintptr_t)d_sums & 7u) return STG_E_ALIGN;
-    if (a.flags & ~STG_PPO_CLIP_VF) return STG_E_ENUM;
-    return stg::ppo_launch<stg::kFoldRaw>(a, d_sums, (cudaStream_t)stream);
+    if (int rc = ppo_check_flags<kLoss>(a)) return rc;
+    return ppo_launch<kLoss, kFoldRaw>(a, d_sums, (cudaStream_t)stream);
+}
+
+}  // namespace stg
+
+extern "C" int stg_policy_ppo_grad_f32(const StgPpoArgs* args, void* stream) {
+    return stg::ppo_grad_entry<stg::kLossPpo>(args, stream);
+}
+
+extern "C" int stg_policy_ppo_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream) {
+    return stg::ppo_sums_entry<stg::kLossPpo>(args, d_sums, stream);
+}
+
+extern "C" int stg_policy_a2c_grad_f32(const StgPpoArgs* args, void* stream) {
+    return stg::ppo_grad_entry<stg::kLossA2c>(args, stream);
+}
+
+extern "C" int stg_policy_a2c_sums_f32(const StgPpoArgs* args, double* d_sums, void* stream) {
+    return stg::ppo_sums_entry<stg::kLossA2c>(args, d_sums, stream);
 }
 
 extern "C" int stg_policy_ppo_finish_f32(const StgPpoArgs* args, const double* d_sums, int32_t ranks, void* stream) {

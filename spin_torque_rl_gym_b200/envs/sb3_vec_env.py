@@ -304,10 +304,7 @@ class RolloutCollector:
         newly allocated tensors (one allocation per batch, split into the six fields), so batches kept by the caller are
         never overwritten; iterating never synchronises with the host. Needs store_values=True, store_observations=True
         and compute_returns_and_advantage() after the last collect(); the arguments are checked when get() is called."""
-        if not (self.store_values and self.store_observations):
-            raise ValueError("get() needs a collector with store_values=True and store_observations=True")
-        if not self._advantages_computed:
-            raise RuntimeError("get() needs compute_returns_and_advantage() after the last collect()")
+        self._check_get()
         total = self.n_steps * self.env.num_envs
         batch_size = total if batch_size is None else int(batch_size)
         if batch_size <= 0:
@@ -315,6 +312,26 @@ class RolloutCollector:
         keys = minibatch_round_keys(self.env.rng_seed, self.env.env_offset, self._epoch)
         self._epoch += 1
         return self._minibatches(keys, batch_size)
+
+    def _check_get(self) -> None:
+        if not (self.store_values and self.store_observations):
+            raise ValueError("get() needs a collector with store_values=True and store_observations=True")
+        if not self._advantages_computed:
+            raise RuntimeError("get() needs compute_returns_and_advantage() after the last collect()")
+
+    def rollout_samples(self) -> RolloutBufferSamples:
+        """The whole stored rollout as one `RolloutBufferSamples` of flat views: n_steps * num_envs rows in (step, env) order
+        (row t * num_envs + i is env i at step t), with no copy, no permutation and no launch. The views alias the collector's
+        planes, so the next collect() overwrites them. Preconditions and errors are those of get().
+
+        This is A2C's batch. SB3's A2C.train() iterates `get(batch_size=None)`, which permutes the rows, but its update is
+        one sum over all of them: a permutation changes only the order of that sum, which K10 fixes anyway, so the rows are
+        used where they lie."""
+        self._check_get()
+        total = self.n_steps * self.env.num_envs
+        return RolloutBufferSamples(self.observations.view(total, _lib.OBS_DIM), self.actions.view(total, 2),
+                                    self.values.view(total), self.log_probs.view(total), self.advantages.view(total),
+                                    self.returns.view(total))
 
     def _minibatches(self, keys: List[int], batch_size: int) -> Iterator[RolloutBufferSamples]:
         env = self.env

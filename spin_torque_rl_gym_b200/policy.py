@@ -5,7 +5,8 @@ Box action (net_arch pi=[64, 64], vf=[64, 64], tanh, FlattenExtractor, DiagGauss
 log_std), so SB3 state dicts load into it and back. Its `forward` and `predict_values`, which a rollout calls over all N envs
 every step, run as single launches of stg_policy_act_f32 / stg_policy_value_f32 (include/stg.h); `evaluate_actions` is plain
 torch with autograd. `ppo_backward` computes SB3's PPO.train() loss of a minibatch and writes every parameter's gradient in
-one launch of stg_policy_ppo_grad_f32 plus a fold (K10)."""
+one launch of stg_policy_ppo_grad_f32 plus a fold (K10); `a2c_backward` does the same for SB3's A2C.train() loss with K10's
+A2C instance (stg_policy_a2c_grad_f32)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -48,9 +49,22 @@ class PPOLosses(NamedTuple):
     clip_fraction: torch.Tensor
 
 
+class A2CLosses(NamedTuple):
+    """The losses of one A2C update with Stable-Baselines3's A2C.train() definitions, each a 0-d float32 tensor on the
+    device: loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss, policy_loss = -mean(advantages * log_prob),
+    value_loss = mse_loss(returns, values), entropy_loss = -mean(entropy)."""
+    loss: torch.Tensor
+    policy_loss: torch.Tensor
+    value_loss: torch.Tensor
+    entropy_loss: torch.Tensor
+
+
 # the sample planes ppo_backward reads: (RolloutBufferSamples field, trailing shape, required alignment in bytes)
 _PPO_PLANES = (("observations", (_lib.OBS_DIM,), 16), ("actions", (2,), 8), ("old_values", (), 4),
                ("old_log_prob", (), 4), ("advantages", (), 4), ("returns", (), 4))
+# the K10 instance of each loss: (gradient entry point, K12 sums entry point, the planes it does not read)
+_K10_LOSSES = {"ppo": ("stg_policy_ppo_grad_f32", "stg_policy_ppo_sums_f32", ()),
+               "a2c": ("stg_policy_a2c_grad_f32", "stg_policy_a2c_sums_f32", ("old_values", "old_log_prob"))}
 
 
 class MlpExtractor(nn.Module):
@@ -282,21 +296,28 @@ class ActorCriticPolicy(nn.Module):
                 (self.action_net.weight, L["ACT_W"]), (self.action_net.bias, L["ACT_B"]),
                 (self.value_net.weight, L["VAL_W"]), (self.value_net.bias, L["VAL_B"]), (self.log_std, L["LOG_STD"]))
 
-    def _ppo_planes(self, samples):
+    def _ppo_planes(self, samples, loss: str = "ppo"):
+        """(B, the six planes of `samples` in _PPO_PLANES order, checked, with None for those `loss` does not read)."""
+        what = f"{loss}_backward"
         obs = samples.observations
         n = obs.shape[0] if isinstance(obs, torch.Tensor) and obs.dim() == 2 else 0
         if n < 1:
-            raise ValueError("ppo_backward needs samples.observations of shape [B, 12] with B >= 1, got "
+            raise ValueError(f"{what} needs samples.observations of shape [B, 12] with B >= 1, got "
                              f"{tuple(obs.shape) if isinstance(obs, torch.Tensor) else type(obs).__name__}")
-        planes = [getattr(samples, name) for name, _, _ in _PPO_PLANES]
+        skip = _K10_LOSSES[loss][2]
+        planes = [None if name in skip else getattr(samples, name) for name, _, _ in _PPO_PLANES]
         for t, (name, tail, _) in zip(planes, _PPO_PLANES):
+            if name in skip:
+                continue
             if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or tuple(t.shape) != (n,) + tail:
                 got = (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t).__name__
                 raise ValueError(f"samples.{name} must be a float32 tensor of shape {(n,) + tail}, got {got}")
         if obs.device.type != "cuda":
-            raise _lib.StgError("ActorCriticPolicy.ppo_backward needs CUDA tensors (no CPU fallback)")
+            raise _lib.StgError(f"ActorCriticPolicy.{what} needs CUDA tensors (no CPU fallback)")
         dev = self.log_std.device
         for i, (t, (name, _, align)) in enumerate(zip(planes, _PPO_PLANES)):
+            if t is None:
+                continue
             if t.device != dev:
                 raise ValueError(f"samples.{name} is on {t.device}, the policy on {dev}")
             if not t.is_contiguous() or t.data_ptr() % align:
@@ -330,8 +351,31 @@ class ActorCriticPolicy(nn.Module):
         Raises StgError without CUDA, ValueError for an empty batch or planes of the wrong shape, dtype or device."""
         if data_parallel:
             return self._ppo_backward_ranks(samples, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage)
-        n, planes = self._ppo_planes(samples)
+        return self._k10_backward(samples, "ppo", clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage)
+
+    def a2c_backward(self, samples, ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = False,
+                     data_parallel: bool = False) -> A2CLosses:
+        """SB3's A2C.train() loss with the current weights, and the gradient of every parameter: the result of
+        `optimizer.zero_grad(); loss.backward()`, in one launch of stg_policy_a2c_grad_f32 and its fold (K10's A2C instance).
+        The loss is PPO's with the clipped surrogate replaced by `-(advantages * log_prob).mean()` and an unclipped value loss.
+
+        `samples`: a RolloutBufferSamples, in A2C the whole rollout (`RolloutCollector.rollout_samples()`); old_values and
+        old_log_prob are not read. Everything else is ppo_backward's: the plane checks and copies, the advantage normalisation
+        (SB3's, with `normalize_advantage` and B > 1), the repacked weights, `.grad` set to views of the one flat gradient
+        buffer that every call OVERWRITES, no host synchronisation, and `data_parallel=True` (K12) giving the loss and
+        gradient of the union of every rank's rows, bit-identical on every rank. Returns A2CLosses.
+        Raises StgError without CUDA, ValueError for an empty batch or planes of the wrong shape, dtype or device."""
+        if data_parallel:
+            losses = self._ppo_backward_ranks(samples, 0.0, None, ent_coef, vf_coef, normalize_advantage, loss="a2c")
+        else:
+            losses = self._k10_backward(samples, "a2c", 0.0, None, ent_coef, vf_coef, normalize_advantage)
+        return A2CLosses(*losses[:4])
+
+    def _k10_backward(self, samples, loss, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage) -> PPOLosses:
+        """One launch of K10's `loss` instance and its fold on one rank: the six losses, .grad set."""
+        n, planes = self._ppo_planes(samples, loss)
         dev = self.log_std.device
+        entry = _K10_LOSSES[loss][0]
         with _lib.device_guard(torch, dev):
             stats = None
             if normalize_advantage and n > 1:
@@ -341,7 +385,7 @@ class ActorCriticPolicy(nn.Module):
             work = torch.empty(_lib.ppo_work_doubles(n), dtype=torch.float64, device=dev)
             a = self._ppo_args(n, planes, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
             a.d_grad, a.d_losses, a.d_work = self._grad_buffer().data_ptr(), losses.data_ptr(), work.data_ptr()
-            self._launch(_lib.load().stg_policy_ppo_grad_f32, a, "stg_policy_ppo_grad_f32")
+            self._launch(getattr(_lib.load(), entry), a, entry)
         self._set_grads()
         return PPOLosses(*losses.unbind())
 
@@ -360,7 +404,8 @@ class ActorCriticPolicy(nn.Module):
         a = _lib.StgPpoArgs()
         a.d_weights = self.pack_weights().data_ptr()
         if planes is not None:
-            a.d_obs, a.d_action, a.d_old_value, a.d_old_log_prob, a.d_advantage, a.d_return = (t.data_ptr() for t in planes)
+            a.d_obs, a.d_action, a.d_old_value, a.d_old_log_prob, a.d_advantage, a.d_return = (
+                None if t is None else t.data_ptr() for t in planes)
         a.d_adv_stats = None if stats is None else stats.data_ptr()
         cr = float(clip_range)
         a.clip_range, a.ratio_lo, a.ratio_hi = cr, 1.0 - cr, 1.0 + cr     # rounded to float32 as torch.clamp does
@@ -372,33 +417,35 @@ class ActorCriticPolicy(nn.Module):
         return a
 
     # ---- K12 -----------------------------------------------------------------------------------------------------------------
-    def _ppo_backward_ranks(self, samples, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage) -> PPOLosses:
-        """ppo_backward(data_parallel=True): moments -> all_gather -> merge -> sums -> all_gather -> finish, on the current
-        stream of the policy's device."""
+    def _ppo_backward_ranks(self, samples, clip_range, clip_range_vf, ent_coef, vf_coef, normalize_advantage,
+                            loss: str = "ppo") -> PPOLosses:
+        """ppo_backward / a2c_backward(data_parallel=True): moments -> all_gather -> merge -> sums of K10's `loss` instance ->
+        all_gather -> finish, on the current stream of the policy's device."""
         from .parallel import all_gather_moments, world_size
-        n, _ = self._ppo_planes(samples)
+        n, _ = self._ppo_planes(samples, loss)
         dev = self.log_std.device
         with _lib.device_guard(torch, dev), torch.cuda.stream(torch.cuda.current_stream(dev)):
             stats = None
             if normalize_advantage and n * world_size() > 1:
                 stats = _adv_stats(all_gather_moments(_adv_moments(samples.advantages)))
-            sums = self._ppo_sums(samples, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
+            sums = self._ppo_sums(samples, stats, clip_range, clip_range_vf, ent_coef, vf_coef, loss=loss)
             return self._ppo_finish(all_gather_moments(sums), ent_coef, vf_coef)
 
     def _ppo_sums(self, samples, stats, clip_range: float = 0.2, clip_range_vf: Optional[float] = None,
-                  ent_coef: float = 0.0, vf_coef: float = 0.5):
-        """The unscaled FP64 sums of this part of a minibatch (stg_policy_ppo_sums_f32): a float64 [STG_PPO_PART] tensor.
-        `stats`: the float32 [2] (mean, std) to normalise the advantages with, or None."""
-        n, planes = self._ppo_planes(samples)
+                  ent_coef: float = 0.0, vf_coef: float = 0.5, loss: str = "ppo"):
+        """The unscaled FP64 sums of this part of a minibatch (stg_policy_ppo_sums_f32, or stg_policy_a2c_sums_f32 for
+        loss="a2c"): a float64 [STG_PPO_PART] tensor. `stats`: the float32 [2] (mean, std) to normalise the advantages with,
+        or None."""
+        n, planes = self._ppo_planes(samples, loss)
+        entry = _K10_LOSSES[loss][1]
         dev = self.log_std.device
         with _lib.device_guard(torch, dev):
             sums = torch.empty(_lib.PPO_PART, dtype=torch.float64, device=dev)
             work = torch.empty(_lib.ppo_work_doubles(n), dtype=torch.float64, device=dev)
             a = self._ppo_args(n, planes, stats, clip_range, clip_range_vf, ent_coef, vf_coef)
             a.d_work = work.data_ptr()
-            _lib.check(_lib.load().stg_policy_ppo_sums_f32(C.byref(a), sums.data_ptr(),
-                                                           torch.cuda.current_stream(dev).cuda_stream),
-                       "stg_policy_ppo_sums_f32")
+            _lib.check(getattr(_lib.load(), entry)(C.byref(a), sums.data_ptr(), torch.cuda.current_stream(dev).cuda_stream),
+                       entry)
         return sums
 
     def _ppo_finish(self, sums, ent_coef: float = 0.0, vf_coef: float = 0.5) -> PPOLosses:

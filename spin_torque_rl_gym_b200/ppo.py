@@ -3,30 +3,20 @@ RolloutCollector with ActorCriticPolicy (K9), GAE (K6), shuffled minibatches (K7
 the clipped Adam step with its device-side target_kl gate (K11, ClippedAdam)."""
 from __future__ import annotations
 
-import math
-from typing import Any, Callable, Dict, List, Optional, Union
+from typing import Any, Dict, Optional, Union
 
 import torch
 
 from . import _lib
 from .envs import RolloutCollector
+from .on_policy import OnPolicyAlgorithm, Schedule, _schedule
 from .optim import ClippedAdam
-from .parallel import all_gather_moments, all_reduce_stats, episode_metrics, world_size
-from .policy import ActorCriticPolicy, _adv_moments
+from .policy import ActorCriticPolicy
 
-Schedule = Union[float, Callable[[float], float]]
 _LOG = _lib.ADAM_LOG_SLOTS
 
 
-def _schedule(value: Optional[Schedule]) -> Optional[Callable[[float], float]]:
-    """SB3's get_schedule_fn: a callable of progress_remaining is kept, a number becomes a constant one."""
-    if value is None or callable(value):
-        return value
-    v = float(value)
-    return lambda _: v
-
-
-class PPO:
+class PPO(OnPolicyAlgorithm):
     """`PPO(policy, env, learning_rate=3e-4, n_steps=2048, batch_size=64, n_epochs=10, gamma=0.99, gae_lambda=0.95,
     clip_range=0.2, clip_range_vf=None, normalize_advantage=True, ent_coef=0.0, vf_coef=0.5, max_grad_norm=0.5,
     target_kl=None, seed=None, policy_kwargs=None, data_parallel=False)`: SB3's PPO signature and defaults for a
@@ -65,29 +55,15 @@ class PPO:
                  ent_coef: float = 0.0, vf_coef: float = 0.5, max_grad_norm: Optional[float] = 0.5,
                  target_kl: Optional[float] = None, seed: Optional[int] = None, policy_kwargs: Optional[Dict[str, Any]] = None,
                  data_parallel: bool = False):
-        ranks = world_size()
-        if ranks > 1 and not data_parallel:
-            raise NotImplementedError("PPO(data_parallel=False) trains on one rank; under a process group of world size "
-                                      f"{ranks} pass data_parallel=True to train one policy across the ranks")
+        ranks = self._ranks(data_parallel)
         if n_steps < 1 or n_epochs < 1 or batch_size < 1:
             raise ValueError(f"n_steps, n_epochs and batch_size must be positive, got {n_steps}, {n_epochs}, {batch_size}")
         if normalize_advantage and batch_size < 2:
             raise ValueError("batch_size must be greater than 1 with normalize_advantage=True (the advantage std of one sample "
                              "is NaN)")
-        if isinstance(policy, str):
-            if policy != "MlpPolicy":
-                raise ValueError(f"the only policy name is 'MlpPolicy', got {policy!r}")
-            if seed is not None:
-                torch.manual_seed(seed)
-            policy = ActorCriticPolicy(env, seed=seed, **(policy_kwargs or {}))
-        elif not isinstance(policy, ActorCriticPolicy):
-            raise ValueError(f"policy must be 'MlpPolicy' or an ActorCriticPolicy, got {type(policy).__name__}")
-        elif policy_kwargs:
-            raise ValueError("policy_kwargs apply to 'MlpPolicy' only")
-        elif policy.num_envs != env.num_envs or policy.log_std.device != torch.device(env.device):
-            raise ValueError("the policy was built for another env (device or num_envs differ)")
+        policy = self._policy(policy, env, seed, policy_kwargs)
         if data_parallel:
-            _check_data_parallel(env, batch_size, ranks)
+            self._check_data_parallel(env, ranks, batch_size)
         self.data_parallel, self.ranks = bool(data_parallel), ranks if data_parallel else 1
         self.env, self.policy = env, policy
         self.n_steps, self.batch_size, self.n_epochs = int(n_steps), int(batch_size), int(n_epochs)
@@ -101,55 +77,12 @@ class PPO:
         dev = policy.log_std.device
         self._log = torch.zeros(_lib.ADAM_LOG, dtype=torch.float64, device=dev)
         self._gate = torch.ones(1, dtype=torch.int32, device=dev)
-        self.num_timesteps = 0
-        self._n_updates = 0
-        self._total_timesteps = 0
-        self._current_progress_remaining = 1.0
-        if self.ranks > 1:
-            self._synchronise_ranks()
-        self._last_stats = all_reduce_stats(env.stats_tensor())
-        self.log_history: List[Dict[str, float]] = []
+        self._start()
 
-    def _synchronise_ranks(self) -> None:
-        """Data-parallel start-up: check that the ranks agree on num_envs, batch_size and the policy seed, then broadcast
-        rank 0's parameters and optimiser state."""
-        import torch.distributed as dist
-        pol, opt = self.policy, self.policy.optimizer
-        seed = pol.seed - (1 << 64) if pol.seed >= 1 << 63 else pol.seed          # the 64-bit seed as an int64
-        mine = torch.tensor([self.env.num_envs, self.batch_size, seed], dtype=torch.int64, device=pol.log_std.device)
-        every = all_gather_moments(mine).cpu()
-        if not bool((every == every[0]).all()):
-            raise ValueError("data-parallel PPO needs the same num_envs, batch_size and policy seed on every rank, got "
-                             f"{every.tolist()} (rows: ranks)")
-        with torch.no_grad():
-            for t in [p.data for p in pol.parameters()] + [opt._exp_avg, opt._exp_avg_sq, opt._step_count]:
-                dist.broadcast(t, src=0)
+    _NAME = "PPO"
 
-    def learn(self, total_timesteps: int, reset_num_timesteps: bool = True) -> "PPO":
-        """SB3's learn(): until num_timesteps reaches total_timesteps, collect n_steps x num_envs samples on the fused path,
-        update progress_remaining, compute GAE and train(). With reset_num_timesteps=False, total_timesteps counts from the
-        current num_timesteps, as in SB3."""
-        if reset_num_timesteps:
-            self.num_timesteps = 0
-        else:
-            total_timesteps += self.num_timesteps
-        self._total_timesteps = total_timesteps
-        iteration = 0
-        col = self.rollout_buffer
-        while self.num_timesteps < total_timesteps:
-            stats = col.collect(self.policy)
-            self.num_timesteps += self.n_steps * self.env.num_envs * self.ranks
-            iteration += 1
-            self._current_progress_remaining = 1.0 - float(self.num_timesteps) / float(total_timesteps)
-            col.compute_returns_and_advantage(self.gamma, self.gae_lambda)
-            rollout = episode_metrics({k: stats[k] - self._last_stats[k] for k in _lib.STAT_NAMES})
-            self._last_stats = stats
-            logs = self.train()
-            for k in ("success_rate", "mean_episode_length", "mean_reward", "episodes"):
-                logs[f"rollout/{k}"] = rollout[k]
-            logs["time/iterations"] = iteration
-            logs["time/total_timesteps"] = self.num_timesteps
-        return self
+    def _rank_agreement(self) -> Dict[str, int]:
+        return {"num_envs": self.env.num_envs, "batch_size": self.batch_size, "policy seed": self._seed_int64()}
 
     def train(self) -> Dict[str, float]:
         """SB3's train() over the collected rollout: n_epochs epochs of get(batch_size) minibatches (get(batch_size // G)
@@ -174,14 +107,8 @@ class PPO:
             self._n_updates += 1
             if self.target_kl is not None and int(gate.item()) == 0:
                 break
+        explained_var = self._rollout_explained_variance()
         with torch.no_grad():
-            values, returns = col.values.reshape(-1), col.returns.reshape(-1)
-            if self.data_parallel:
-                moments = all_gather_moments(torch.cat([_adv_moments(returns), _adv_moments(returns - values)]))
-                explained_var = _explained_variance(moments.reshape(-1, 2, _lib.PPO_ADV_MOMENTS))
-            else:
-                var_y = returns.var(correction=0)
-                explained_var = torch.where(var_y == 0, math.nan, 1 - (returns - values).var(correction=0) / var_y)
             count = log[_LOG["COUNT"]]
             row = torch.stack([log[_LOG["ENTROPY"]] / count, log[_LOG["PG"]] / count, log[_LOG["VALUE"]] / count,
                                log[_LOG["EPOCH_KL"]] / log[_LOG["EPOCH_COUNT"]], log[_LOG["CLIP"]] / count,
@@ -197,26 +124,3 @@ class PPO:
         logs["train/learning_rate"] = lr
         self.log_history.append(logs)
         return logs
-
-    def predict(self, obs, deterministic: bool = False):
-        """The policy's predict: (env actions, None)."""
-        return self.policy.predict(obs, deterministic=deterministic)
-
-
-def _check_data_parallel(env, batch_size: int, ranks: int) -> None:
-    """The ValueErrors of PPO(data_parallel=True) that need no collective."""
-    from .envs.vec_normalize import VecNormalize
-    if batch_size % ranks:
-        raise ValueError(f"data-parallel PPO needs batch_size divisible by the world size {ranks}, got {batch_size}")
-    if isinstance(env, VecNormalize) and not env._syncing():
-        raise ValueError("data-parallel PPO needs a VecNormalize that shares its statistics across the ranks (sync=None or "
-                         "True), or the ranks would normalise their observations differently")
-
-
-def _explained_variance(moments):
-    """1 - Var(returns - values) / Var(returns) (population variances, NaN when Var(returns) is 0) from moments [G, 2, 3]:
-    per rank the FP64 (n, mean, M2) of the returns and of returns - values. Each is folded in rank order with K12's merge
-    (stg_ppo_adv_merge_f32 gives torch's std with correction 1, whose square ratio is the ratio of the M2)."""
-    from .policy import _adv_stats
-    std_y, std_d = _adv_stats(moments[:, 0])[1].double(), _adv_stats(moments[:, 1])[1].double()
-    return torch.where(std_y == 0, math.nan, 1 - (std_d * std_d) / (std_y * std_y))
