@@ -107,10 +107,14 @@ STG_HD ArrayAction array_parse_action(const StgArrayParams& p, const float* act)
         cur = (double)act[1];
         dur = (double)act[2];
     }
-    a.cur = fmin(fmax(cur, -p.max_current), p.max_current);
-    a.dur = fmin(fmax(dur, 1e-12), p.max_duration);
+    // np.clip keeps NaN (both comparisons are false); fmin/fmax would drop it. A NaN current then drives nothing and costs no
+    // energy (|NaN| > 1e-12 is false), and a NaN duration propagates through the dynamics and the energy, as in the reference.
+    auto clip = [](double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); };
+    a.cur = clip(cur, -p.max_current, p.max_current);
+    a.dur = clip(dur, 1e-12, p.max_duration);
     const float a0 = act[0];
-    auto clip_idx = [](float v, int hi) {          // int(np.clip(action[0], 0, hi)) on a float32 scalar
+    // int(np.clip(action[0], 0, hi)) on a float32 scalar. The reference raises on a NaN index; a kernel cannot, so it takes 0.
+    auto clip_idx = [](float v, int hi) {
         float c = fminf(fmaxf(v, 0.0f), (float)hi);
         if (!(c == c)) c = 0.0f;
         return (int)c;

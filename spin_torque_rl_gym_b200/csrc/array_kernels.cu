@@ -505,6 +505,20 @@ static int check_array_args(const StgArrayStepArgs& a) {
     return STG_OK;
 }
 
+// A launch may use 48 KB of static plus dynamic shared memory without the opt-in, so the kernel's static part counts too
+// (the one-warp step kernel's 80 B push 1x877 = 49,112 B of dynamic shared memory over the line). The static size is a
+// property of the compiled kernel: it is queried once per kernel and kept in *static_bytes (-1 = not yet known).
+static int opt_in_shared_memory(const void* kernel, size_t dynamic_bytes, int* static_bytes) {
+    if (*static_bytes < 0) {
+        cudaFuncAttributes fa;
+        const cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+        if (e != cudaSuccess) return (int)e;
+        *static_bytes = (int)fa.sharedSizeBytes;
+    }
+    if (dynamic_bytes + (size_t)*static_bytes <= 48 * 1024) return STG_OK;
+    return (int)cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic_bytes);
+}
+
 extern "C" int stg_array_step_f64(const StgArrayStepArgs* args, void* stream) {
     if (!args) return STG_E_NULL;
     const StgArrayStepArgs& a = *args;
@@ -514,11 +528,6 @@ extern "C" int stg_array_step_f64(const StgArrayStepArgs* args, void* stream) {
     if (a.action_stride < (a.params.action_mode == STG_ARRAY_GLOBAL ? 2 : 3)) return STG_E_SIZE;
     if (a.n_arrays == 0) return STG_OK;
     const int nd = a.params.n_rows * a.params.n_cols;
-    const size_t smem = sizeof(double) * 7 * (size_t)nd;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(stg::array_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-    }
     // four arrays per warp, eight lanes each. The observation rows are written as 8-byte words (6 f32 per device = 3 words),
     // so d_obs / d_final_obs must be 8-byte aligned for this kernel; anything else takes the one-warp kernel.
     const auto aligned = [](const void* q, uintptr_t n) { return (reinterpret_cast<uintptr_t>(q) & (n - 1)) == 0; };
@@ -543,6 +552,10 @@ extern "C" int stg_array_step_f64(const StgArrayStepArgs* args, void* stream) {
         else stg::array_step_kernel8<0, false><<<grid, 32, smem8, (cudaStream_t)stream>>>(a);
         return (int)cudaGetLastError();
     }
+    const size_t smem = sizeof(double) * 7 * (size_t)nd;
+    static int static_smem = -1;
+    rc = opt_in_shared_memory((const void*)stg::array_step_kernel, smem, &static_smem);
+    if (rc != STG_OK) return rc;
     stg::array_step_kernel<<<(unsigned)a.n_arrays, stg::kArrayBlock, smem, (cudaStream_t)stream>>>(a);
     return (int)cudaGetLastError();
 }
@@ -555,10 +568,9 @@ extern "C" int stg_array_reset(const StgArrayStepArgs* args, const uint8_t* d_ma
     if (a.n_arrays == 0) return STG_OK;
     const int nd = a.params.n_rows * a.params.n_cols;
     const size_t smem = sizeof(double) * 6 * (size_t)nd;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(stg::array_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-    }
+    static int static_smem = -1;
+    rc = opt_in_shared_memory((const void*)stg::array_reset_kernel, smem, &static_smem);
+    if (rc != STG_OK) return rc;
     stg::array_reset_kernel<<<(unsigned)a.n_arrays, stg::kArrayBlock, smem, (cudaStream_t)stream>>>(a, d_mask, d_pattern0);
     return (int)cudaGetLastError();
 }

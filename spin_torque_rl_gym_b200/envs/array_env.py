@@ -45,6 +45,36 @@ def compute_coupling_matrix(n_rows: int, n_cols: int, coupling_strength: float, 
     return out
 
 
+def array_params(array_size: Tuple[int, int], device_type: str, device_params: Dict[str, Any], action_mode: str,
+                 max_steps: int, max_current: float, max_duration: float, success_threshold: float,
+                 energy_penalty_weight: float) -> _lib.StgArrayParams:
+    """K3's parameter block (StgArrayParams) for one array configuration: the device's field and resistance constants
+    as the reference's device classes derive them from device_params."""
+    p = _lib.StgArrayParams()
+    p.n_rows, p.n_cols = array_size
+    p.action_mode = _lib.ARRAY_MODES[action_mode]
+    p.device_kind = _params.DEVICE_KINDS[device_type]
+    p.max_steps = int(max_steps)
+    ms = float(device_params.get("saturation_magnetization", 800e3))
+    p.hk = 2 * float(device_params.get("uniaxial_anisotropy", 1e6)) / (MU0 * ms)
+    p.saturation_magnetization = ms
+    p.easy_axis = _lib.c_double3(*np.asarray(device_params.get("easy_axis", [0, 0, 1]), dtype=float))
+    st = _params.make_param_struct(device_type, device_params, max_steps=max_steps, max_current=max_current,
+                                   max_duration=max_duration, temperature=300.0, thermal=False,
+                                   success_threshold=success_threshold, energy_penalty_weight=energy_penalty_weight)
+    if p.device_kind != _lib.DEV_STT:
+        ar = float(device_params.get("aspect_ratio", 1.0))
+        nx, ny = (1.0 / (1.0 + ar), ar / (1.0 + ar)) if ar >= 1.0 else (ar / (1.0 + ar), 1.0 / (1.0 + ar))
+        p.demag_n = _lib.c_double3(nx, ny, 1.0 - nx - ny)
+    ref = np.asarray(device_params.get("reference_magnetization", [0, 0, 1]), dtype=float)
+    p.reference_magnetization = _lib.c_double3(*(ref / np.linalg.norm(ref)))
+    p.resistance_parallel, p.resistance_antiparallel = st.resistance_parallel, st.resistance_antiparallel
+    p.series_resistance, p.area = st.series_resistance, st.area
+    p.max_current, p.max_duration = float(max_current), float(max_duration)
+    p.success_threshold, p.energy_penalty_weight = float(success_threshold), float(energy_penalty_weight)
+    return p
+
+
 class SpinTorqueArrayVectorEnv:
     metadata = {"render_modes": [], "autoreset_mode": "same_step"}
 
@@ -99,30 +129,9 @@ class SpinTorqueArrayVectorEnv:
         _params.check_device_constructible(device_type, device_params)
         self.device_params = dict(device_params)
 
-        p = _lib.StgArrayParams()
-        p.n_rows, p.n_cols = self.n_rows, self.n_cols
-        p.action_mode = _lib.ARRAY_MODES[action_mode]
-        p.device_kind = _params.DEVICE_KINDS[device_type]
-        p.max_steps = self.max_steps
-        ms = float(device_params.get("saturation_magnetization", 800e3))
-        p.hk = 2 * float(device_params.get("uniaxial_anisotropy", 1e6)) / (MU0 * ms)
-        p.saturation_magnetization = ms
-        p.easy_axis = _lib.c_double3(*np.asarray(device_params.get("easy_axis", [0, 0, 1]), dtype=float))
-        st = _params.make_param_struct(device_type, device_params, max_steps=self.max_steps, max_current=self.max_current,
-                                       max_duration=self.max_duration, temperature=300.0, thermal=False,
-                                       success_threshold=self.success_threshold,
-                                       energy_penalty_weight=self.energy_penalty_weight)
-        if p.device_kind != _lib.DEV_STT:
-            ar = float(device_params.get("aspect_ratio", 1.0))
-            nx, ny = (1.0 / (1.0 + ar), ar / (1.0 + ar)) if ar >= 1.0 else (ar / (1.0 + ar), 1.0 / (1.0 + ar))
-            p.demag_n = _lib.c_double3(nx, ny, 1.0 - nx - ny)
-        ref = np.asarray(device_params.get("reference_magnetization", [0, 0, 1]), dtype=float)
-        p.reference_magnetization = _lib.c_double3(*(ref / np.linalg.norm(ref)))
-        p.resistance_parallel, p.resistance_antiparallel = st.resistance_parallel, st.resistance_antiparallel
-        p.series_resistance, p.area = st.series_resistance, st.area
-        p.max_current, p.max_duration = self.max_current, self.max_duration
-        p.success_threshold, p.energy_penalty_weight = self.success_threshold, self.energy_penalty_weight
-        self._params_struct = p
+        self._params_struct = array_params(self.array_size, device_type, device_params, action_mode, self.max_steps,
+                                           self.max_current, self.max_duration, self.success_threshold,
+                                           self.energy_penalty_weight)
 
         N, D, dev, f64 = self.num_envs, self.n_devices, self.device, torch.float64
         if target_pattern is None:

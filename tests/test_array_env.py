@@ -32,20 +32,12 @@ def test_oracle_bit_exact(name):
 
 def _host_env(size, mode, kw):
     """StgArrayStepArgs over NumPy buffers driven through tests/hostsim (same helpers as the CUDA kernel)."""
-    from spin_torque_rl_gym_b200.envs.array_env import compute_coupling_matrix
+    from spin_torque_rl_gym_b200.envs.array_env import array_params, compute_coupling_matrix
     from spin_torque_rl_gym_b200 import params as P
     from tests.hostsim.harness import lib
-    dp = P.default_device_parameters("stt_mram")
     D = size[0] * size[1]
-    p = _lib.StgArrayParams()
-    p.n_rows, p.n_cols, p.action_mode, p.device_kind = size[0], size[1], _lib.ARRAY_MODES[mode], 0
-    p.max_steps = kw.get("max_steps", 200)
-    p.hk = 2 * dp["uniaxial_anisotropy"] / (4 * np.pi * 1e-7 * dp["saturation_magnetization"])
-    p.saturation_magnetization = dp["saturation_magnetization"]
-    p.easy_axis = _lib.c_double3(0, 0, 1)
-    p.reference_magnetization = _lib.c_double3(0, 0, 1)
-    p.resistance_parallel, p.resistance_antiparallel, p.area = 1e3, 2e3, dp["area"]
-    p.max_current, p.max_duration, p.success_threshold, p.energy_penalty_weight = 2e6, 5e-9, 0.9, 0.1
+    p = array_params(size, "stt_mram", P.default_device_parameters("stt_mram"), mode, kw.get("max_steps", 200), 2e6, 5e-9,
+                     0.9, 0.1)
     coup = compute_coupling_matrix(size[0], size[1], kw.get("coupling_strength", 0.1), kw.get("coupling_type", "dipolar"))
     st = dict(coup=np.ascontiguousarray(coup), pattern=np.zeros((1, D, 3)), target=np.zeros((1, D, 3)),
               te=np.zeros(1), sc=np.zeros(1, np.int32), ep=np.zeros(1, np.int32), obs=np.zeros((1, D, 6), np.float32),
